@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # CPU arm: the reference algorithm on host cores
+    python bench.py --steps K --warmup W --dump-outputs DIR   # + DIR/codes.npy: the codes of the last timed step
 
 A step = one full pass of index generation (generate_indices.py:85-128: encoder -> 4-level residual
 quantisation -> up to 20 rounds of sort/unique + per-group Sinkhorn) over the whole synthetic item set.
@@ -295,6 +296,27 @@ def workload_config(gpus, items, steps, warmup, cpu_sample=None):
 
 
 # ----------------------------------------------------------------------------- GPU arm
+DUMP_BYTES = 64 << 20        # --dump-outputs: bytes written in all (all ranks together)
+
+
+def dump_outputs(out_dir, arrays, budget):
+    """Each array as out_dir/<name>.npy, float64 arrays as float64 and everything else as float32 (codes < 2^24 are exact).
+    Arrays larger than `budget` bytes in all keep a fixed, seeded sample of their rows (the same rows for the same
+    shape in every run), written in ascending row order with the row numbers beside them as <name>_rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v.detach().cpu() if hasattr(v, "detach") else v) for k, v in arrays.items()}
+    arrays = {k: v.astype(np.float64 if v.dtype == np.float64 else np.float32) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    with_rows = sum(v.nbytes + 8 * v.shape[0] for v in arrays.values() if v.ndim)
+    for name, v in arrays.items():
+        if total > budget and v.ndim and v.shape[0] > 1:
+            keep = max(1, int(v.shape[0] * budget / with_rows))
+            rows = np.sort(np.random.default_rng(SEED_X).choice(v.shape[0], keep, replace=False))
+            v = v[rows]
+            np.save(os.path.join(out_dir, f"{name}_rows.npy"), rows.astype(np.float64))
+        np.save(os.path.join(out_dir, f"{name}.npy"), v)
+
+
 def run_gpu_arm(a):
     import torch
     import torch.distributed as dist
@@ -372,6 +394,8 @@ def run_gpu_arm(a):
         torch.cuda.profiler.stop()
     ms_total = e0.elapsed_time(e1)
     clocks = sampler.stop() if sampler else None
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"codes" if world == 1 else f"codes_rank{rank}": codes}, DUMP_BYTES // world)
     launches = ops.launch_count() - launches0
     prof = ops.profile_collect()
     ops.profile_enable(False)
@@ -747,7 +771,14 @@ def main():
                     help="c3: index generation, 4 x 256 codes (default; BASELINE configs[2] / [3]); c5: 4 x 8192 codes, e_dim 256 "
                          "(configs[4]; --items defaults to 100000); c2: the training epoch (configs[1])")
     ap.add_argument("--bn", action="store_true", help="c2: BatchNorm in the encoder / decoder (what `run.sh --bn False` really trains)")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="c3 / c5: write the codes of the last timed step as DIR/codes.npy (float32; DIR/codes_rank<r>.npy per rank "
+                         "for N > 1), at most 64 MB in all: larger tables keep a fixed, seeded sample of rows (DIR/<name>_rows.npy)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl == "reference" or a.config == "c2"):
+        ap.error("--dump-outputs applies to the GPU arm of --config c3 / c5")
     a.warmup = max(a.warmup, 0)
     set_config(a.config)
     if a.config == "c5":

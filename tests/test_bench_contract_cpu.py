@@ -5,6 +5,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import torch
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -48,3 +51,26 @@ def test_reference_arm_runs_the_staged_reference_script(tmp_path):
     assert line["impl"] == "reference" and line["cpu_baseline"]["kind"] == ("reference" if staged else "port")
     assert line["value"] > 0 and line["e2e"]["h2d_bytes_per_step"] == 0 and line["config"]["reference_sample_items"] == 256
     assert line["cpu_baseline"]["cores"] >= 1
+
+
+def test_dump_outputs_writes_float_arrays_within_the_budget(tmp_path):
+    """--dump-outputs: codes come back exactly as float32; above the byte budget the same seeded rows are kept in every run."""
+    b = _bench()
+    codes = (np.arange(4000, dtype=np.int64) * 7919 % 256).reshape(1000, 4)
+    b.dump_outputs(str(tmp_path / "all"), {"codes": codes}, 1 << 20)
+    got = np.load(tmp_path / "all" / "codes.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, codes) and not (tmp_path / "all" / "codes_rows.npy").exists()
+    for run in ("s1", "s2"):
+        b.dump_outputs(str(tmp_path / run), {"codes": torch.from_numpy(codes)}, 6000)
+    rows = np.load(tmp_path / "s1" / "codes_rows.npy")
+    got = np.load(tmp_path / "s1" / "codes.npy")
+    assert rows.dtype == np.float64 and got.nbytes + rows.nbytes <= 6000 and len(rows) == 250 and (np.diff(rows) > 0).all()
+    assert np.array_equal(got, codes[rows.astype(np.int64)])
+    assert np.array_equal(rows, np.load(tmp_path / "s2" / "codes_rows.npy")) and np.array_equal(got, np.load(tmp_path / "s2" / "codes.npy"))
+
+
+def test_bench_rejects_zero_steps_and_dumps_outside_the_gpu_arm(tmp_path):
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)], ["--config", "c2", "--dump-outputs", str(tmp_path)]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True, timeout=120,
+                           env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), cwd=str(tmp_path))
+        assert r.returncode == 2 and ("--steps" in r.stderr or "--dump-outputs" in r.stderr), r.stderr[-300:]
