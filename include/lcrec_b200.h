@@ -54,6 +54,14 @@ int64_t lcrec_mlp_workspace_bytes(const lcrec_mlp_t* mlp, int64_t n_rows);
  * (acts[n_layers-1] may alias y).  Used by the training path to keep activations. */
 int lcrec_mlp_forward(lcrec_mlp_t* mlp, const float* x, int64_t n_rows, float* y,
                       float* const* acts, void* workspace, int64_t workspace_bytes, void* stream);
+/* The same with x of element type `dtype`: 0 = fp32, 1 = fp16, 2 = bf16 (the codes of lcrec_masked_mean_pool).  Half
+ * inputs are read as they are (no fp32 copy) and converted to fp32 in the layer-1 operand split; the result is
+ * bit-identical to lcrec_mlp_forward on the input upcast to fp32.  x: (n_rows, dims[0]) contiguous; any alignment
+ * (a misaligned base falls back to scalar loads).  dtype outside {0, 1, 2}: LCREC_ERR_ARG, before anything touches the
+ * device.  Half input with engine 0 (tf32 x3): LCREC_ERR_UNSUPPORTED.  lcrec_mlp_forward(...) is
+ * lcrec_mlp_forward_ex(mlp, x, 0, ...). */
+int lcrec_mlp_forward_ex(lcrec_mlp_t* mlp, const void* x, int dtype, int64_t n_rows, float* y,
+                         float* const* acts, void* workspace, int64_t workspace_bytes, void* stream);
 /* accumulation chunk: number of K elements accumulated inside TMEM before the partial sum is
  * folded into fp32 registers with round-to-nearest (0 = whole K in TMEM). */
 int lcrec_mlp_set_acc_chunk(lcrec_mlp_t* mlp, int k_elems);
@@ -317,6 +325,11 @@ int lcrec_sort_codes(const int64_t* codes, int64_t n, int n_levels, const int32_
 
 /* ---- a15: whole index generation, HOST buffers (index/generate_indices.py:85-128) -------
  * x_host: (n, dims[0]) fp32 in pageable or pinned host memory; codes_host: (n, L) int64.
+ * The _ex forms take the embeddings as `const void* x, int dtype` (0 = fp32, 1 = fp16, 2 = bf16, as in
+ * lcrec_mlp_forward_ex): half-precision embeddings are read, and for run_host copied to the device, as they are
+ * (half the bytes of fp32).  Codes and stats are bit-identical to the fp32 entry run on the input upcast to fp32.
+ * dtype outside {0, 1, 2}: LCREC_ERR_ARG, before anything touches the device; half input needs encoder engine 1.
+ * Each fp32 entry is its _ex form with dtype 0.
  * Streams the embeddings to the device in chunks, PASS 0 argmin, then up to max_rounds
  * collision rounds with per-group Sinkhorn on the last level.  stats_host (nullable, 8 int64):
  * [rounds_run, n_unique_final, groups_round1, rows_round1, total_sinkhorn_rows, max_multiplicity,
@@ -333,8 +346,13 @@ int lcrec_indexer_run_device(lcrec_indexer_t* ix, const float* x, int64_t n, int
 /* host-resident input and output */
 int lcrec_indexer_run_host(lcrec_indexer_t* ix, const float* x_host, int64_t n, int max_rounds,
                            int64_t* codes_host, int64_t* stats_host, void* stream);
+int lcrec_indexer_run_device_ex(lcrec_indexer_t* ix, const void* x, int dtype, int64_t n, int max_rounds,
+                                int64_t* codes, int64_t* stats_host, void* stream);
+int lcrec_indexer_run_host_ex(lcrec_indexer_t* ix, const void* x_host, int dtype, int64_t n, int max_rounds,
+                              int64_t* codes_host, int64_t* stats_host, void* stream);
 /* building blocks of the loop, for multi-GPU drivers and tests */
 int lcrec_indexer_pass0(lcrec_indexer_t* ix, const float* x, int64_t n, int64_t row_offset, void* stream);
+int lcrec_indexer_pass0_ex(lcrec_indexer_t* ix, const void* x, int dtype, int64_t n, int64_t row_offset, void* stream);
 int lcrec_indexer_round(lcrec_indexer_t* ix, int64_t n, int64_t* counts_host, void* stream);
 /* The collision rounds alone (generate_indices.py:108-128) on caller-owned device arrays: codes (n, L) int64 updated
  * in place, resid (n, e_dim) = residual entering the last level; n <= max_items.  stats_host as in run_host. */

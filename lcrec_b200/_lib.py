@@ -27,6 +27,7 @@ SIGNATURES = {
     "lcrec_mlp_destroy": (C.c_int, [vp]),
     "lcrec_mlp_workspace_bytes": (i64, [vp, i64]),
     "lcrec_mlp_forward": (C.c_int, [vp, vp, i64, vp, pp, vp, i64, vp]),
+    "lcrec_mlp_forward_ex": (C.c_int, [vp, vp, C.c_int, i64, vp, pp, vp, i64, vp]),
     "lcrec_mlp_set_acc_chunk": (C.c_int, [vp, C.c_int]),
     "lcrec_mlp_set_variant": (C.c_int, [vp, C.c_int]),
     "lcrec_mlp_set_engine": (C.c_int, [vp, C.c_int]),
@@ -76,6 +77,9 @@ SIGNATURES = {
     "lcrec_indexer_run_device": (C.c_int, [vp, vp, i64, C.c_int, vp, C.POINTER(i64), vp]),
     "lcrec_indexer_run_host": (C.c_int, [vp, vp, i64, C.c_int, vp, C.POINTER(i64), vp]),
     "lcrec_indexer_pass0": (C.c_int, [vp, vp, i64, i64, vp]),
+    "lcrec_indexer_run_device_ex": (C.c_int, [vp, vp, C.c_int, i64, C.c_int, vp, C.POINTER(i64), vp]),
+    "lcrec_indexer_run_host_ex": (C.c_int, [vp, vp, C.c_int, i64, C.c_int, vp, C.POINTER(i64), vp]),
+    "lcrec_indexer_pass0_ex": (C.c_int, [vp, vp, C.c_int, i64, i64, vp]),
     "lcrec_indexer_round": (C.c_int, [vp, i64, C.POINTER(i64), vp]),
     "lcrec_indexer_resolve": (C.c_int, [vp, vp, vp, i64, C.c_int, C.POINTER(i64), vp]),
     "lcrec_indexer_set_segments": (C.c_int, [C.c_int]),

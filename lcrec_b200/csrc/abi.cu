@@ -243,14 +243,17 @@ extern "C" int lcrec_indexer_destroy(lcrec_indexer_t* ix) {
 extern "C" int64_t* lcrec_indexer_codes(lcrec_indexer_t* ix) { return ix ? ix->codes : nullptr; }
 extern "C" float* lcrec_indexer_resid(lcrec_indexer_t* ix) { return ix ? ix->resid : nullptr; }
 
-// PASS 0 for rows [row_offset, row_offset + n) (generate_indices.py:85-95)
-extern "C" int lcrec_indexer_pass0(lcrec_indexer_t* ix, const float* x, int64_t n, int64_t row_offset, void* stream) {
+// PASS 0 for rows [row_offset, row_offset + n) (generate_indices.py:85-95); x of element type dtype
+extern "C" int lcrec_indexer_pass0_ex(lcrec_indexer_t* ix, const void* x, int dtype, int64_t n, int64_t row_offset, void* stream) {
+  LC_ARG(dtype_ok(dtype));
   LC_ARG(ix && n >= 0 && row_offset >= 0 && row_offset + n <= ix->max_items);
   if (n == 0) return LCREC_OK;
   LC_ARG(x != nullptr);
+  const int64_t row_bytes = dtype_bytes(dtype) * ix->in_dim;
   for (int64_t s = 0; s < n; s += ix->chunk_rows) {
     const int64_t m = std::min(ix->chunk_rows, n - s);
-    LC_TRY(lcrec_mlp_forward(ix->enc, x + s * ix->in_dim, m, ix->z + s * ix->D, nullptr, ix->mlp_ws, ix->mlp_ws_bytes, stream));
+    LC_TRY(lcrec_mlp_forward_ex(ix->enc, static_cast<const char*>(x) + s * row_bytes, dtype, m, ix->z + s * ix->D, nullptr,
+                                ix->mlp_ws, ix->mlp_ws_bytes, stream));
   }
   {
     ProfScope prof(20, (cudaStream_t)stream);
@@ -259,6 +262,10 @@ extern "C" int lcrec_indexer_pass0(lcrec_indexer_t* ix, const float* x, int64_t 
                              nullptr, stream));
   }
   return LCREC_OK;
+}
+
+extern "C" int lcrec_indexer_pass0(lcrec_indexer_t* ix, const float* x, int64_t n, int64_t row_offset, void* stream) {
+  return lcrec_indexer_pass0_ex(ix, x, kDtypeF32, n, row_offset, stream);
 }
 
 static int g_use_segments = 1;
@@ -490,10 +497,16 @@ extern "C" int lcrec_indexer_round(lcrec_indexer_t* ix, int64_t n, int64_t* coun
 
 extern "C" int lcrec_indexer_run_device(lcrec_indexer_t* ix, const float* x, int64_t n, int max_rounds, int64_t* codes,
                                         int64_t* stats_host, void* stream) {
+  return lcrec_indexer_run_device_ex(ix, x, kDtypeF32, n, max_rounds, codes, stats_host, stream);
+}
+
+extern "C" int lcrec_indexer_run_device_ex(lcrec_indexer_t* ix, const void* x, int dtype, int64_t n, int max_rounds, int64_t* codes,
+                                           int64_t* stats_host, void* stream) {
+  LC_ARG(dtype_ok(dtype));
   LC_ARG(ix && n >= 0 && n <= ix->max_items && max_rounds >= 0);
   cudaStream_t st = (cudaStream_t)stream;
   if (n == 0) { if (stats_host) memset(stats_host, 0, 8 * sizeof(int64_t)); return LCREC_OK; }
-  LC_TRY(lcrec_indexer_pass0(ix, x, n, 0, stream));
+  LC_TRY(lcrec_indexer_pass0_ex(ix, x, dtype, n, 0, stream));
   LC_TRY(indexer_rounds(ix, n, max_rounds, stats_host, st));
   if (codes && codes != ix->codes)
     LC_CUDA(cudaMemcpyAsync(codes, ix->codes, sizeof(int64_t) * n * ix->L, cudaMemcpyDeviceToDevice, st));
@@ -502,6 +515,12 @@ extern "C" int lcrec_indexer_run_device(lcrec_indexer_t* ix, const float* x, int
 
 extern "C" int lcrec_indexer_run_host(lcrec_indexer_t* ix, const float* x_host, int64_t n, int max_rounds,
                                       int64_t* codes_host, int64_t* stats_host, void* stream) {
+  return lcrec_indexer_run_host_ex(ix, x_host, kDtypeF32, n, max_rounds, codes_host, stats_host, stream);
+}
+
+extern "C" int lcrec_indexer_run_host_ex(lcrec_indexer_t* ix, const void* x_host, int dtype, int64_t n, int max_rounds,
+                                         int64_t* codes_host, int64_t* stats_host, void* stream) {
+  LC_ARG(dtype_ok(dtype));
   LC_ARG(ix && n >= 0 && n <= ix->max_items && max_rounds >= 0);
   cudaStream_t st = (cudaStream_t)stream;
   if (n == 0) { if (stats_host) memset(stats_host, 0, 8 * sizeof(int64_t)); return LCREC_OK; }
@@ -514,7 +533,7 @@ extern "C" int lcrec_indexer_run_host(lcrec_indexer_t* ix, const float* x_host, 
       LC_CUDA(cudaMalloc((void**)&ix->stage[i], sizeof(float) * ix->chunk_rows * ix->in_dim));
     }
   }
-  // double-buffered H2D on the copy stream, compute on `st`.  The copies are the bottleneck (55 GB/s of pinned H2D against ~14 M
+  // double-buffered H2D on the copy stream, compute on `st` (the fp32-sized staging buffers also hold a piece of half rows).  The copies are the bottleneck (55 GB/s of pinned H2D against ~14 M
   // items/s of compute), so what is left after the LAST copy lands - that chunk's encoder pass - is pure tail: the last chunk is cut
   // into up to four pieces (>= 8192 rows each) so that only a quarter of it remains to be encoded when the link goes idle.
   std::vector<std::pair<int64_t, int64_t>> pieces;
@@ -526,15 +545,16 @@ extern "C" int lcrec_indexer_run_host(lcrec_indexer_t* ix, const float* x_host, 
     for (int64_t t = 0; t < m0; t += q) pieces.emplace_back(s0 + t, std::min(q, m0 - t));
   }
   const int64_t nchunks = (int64_t)pieces.size();
+  const int64_t row_bytes = dtype_bytes(dtype) * ix->in_dim;
   for (int64_t c = 0; c < nchunks; ++c) {
     const int b = (int)(c & 1);
     const int64_t s = pieces[c].first, m = pieces[c].second;
     if (c >= 2) LC_CUDA(cudaStreamWaitEvent(ix->copy_stream, ix->ev_consumed[b], 0));
-    LC_CUDA(cudaMemcpyAsync(ix->stage[b], x_host + s * ix->in_dim, sizeof(float) * m * ix->in_dim,
+    LC_CUDA(cudaMemcpyAsync(ix->stage[b], static_cast<const char*>(x_host) + s * row_bytes, m * row_bytes,
                             cudaMemcpyHostToDevice, ix->copy_stream));
     LC_CUDA(cudaEventRecord(ix->ev_copied[b], ix->copy_stream));
     LC_CUDA(cudaStreamWaitEvent(st, ix->ev_copied[b], 0));
-    LC_TRY(lcrec_indexer_pass0(ix, ix->stage[b], m, s, stream));
+    LC_TRY(lcrec_indexer_pass0_ex(ix, ix->stage[b], dtype, m, s, stream));
     LC_CUDA(cudaEventRecord(ix->ev_consumed[b], st));
   }
   LC_TRY(indexer_rounds(ix, n, max_rounds, stats_host, st));

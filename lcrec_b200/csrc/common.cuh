@@ -48,6 +48,11 @@ inline void count_launch(int n = 1) { g_launches.fetch_add(n, std::memory_order_
     if (_r != LCREC_OK) return _r;                                                           \
   } while (0)
 
+// element type codes of inputs that may be half precision (the `dtype` arguments of the C ABI)
+constexpr int kDtypeF32 = 0, kDtypeF16 = 1, kDtypeBF16 = 2;
+inline bool dtype_ok(int dtype) { return dtype == kDtypeF32 || dtype == kDtypeF16 || dtype == kDtypeBF16; }
+inline int64_t dtype_bytes(int dtype) { return dtype == kDtypeF32 ? 4 : 2; }
+
 inline int64_t round_up(int64_t x, int64_t m) { return (x + m - 1) / m * m; }
 inline int64_t ceil_div(int64_t x, int64_t m) { return (x + m - 1) / m; }
 

@@ -1,6 +1,7 @@
 // Internal interface between the GEMM translation units (linear_tf32x3.cu, linear_pair.cu).
 #pragma once
 #include <cuda.h>
+#include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
 #include "common.cuh"
@@ -42,8 +43,43 @@ bool argmin_pair_supported(int k, int n_out);
 void set_pair_cluster_cap(int cap);   // 0 = all CTA pairs the device holds
 constexpr int kPairGroup = 256;
 
-// x (rows, k) fp32 -> group-scaled fp16 hi/lo (one pass; scale groups of 256 elements)
-int launch_split_groups(const float* x, int64_t rows, int k, int64_t ldx, __half* hi, __half* lo, int64_t ld_out,
+// x (rows, k) of element type `dtype` (kDtypeF32 / kDtypeF16 / kDtypeBF16; ldx in elements) -> group-scaled fp16 hi/lo
+// (one pass; scale groups of 256 elements)
+int launch_split_groups(const void* x, int dtype, int64_t rows, int k, int64_t ldx, __half* hi, __half* lo, int64_t ld_out,
                         float* inv_scale, int64_t ld_scale, cudaStream_t st);
+
+// Input loads of the operand splits.  Both half formats convert to fp32 exactly, so everything after the load is the
+// arithmetic of the fp32 input.
+__device__ __forceinline__ float to_f32(float v) { return v; }
+__device__ __forceinline__ float to_f32(__half v) { return __half2float(v); }
+__device__ __forceinline__ float to_f32(__nv_bfloat16 v) { return __bfloat162float(v); }
+
+// four consecutive elements at p -> v[0..3]; p 16-byte aligned (fp32) or 8-byte aligned (halves).  STREAM: __ldcs, for
+// an input that is read once.
+template <bool STREAM>
+__device__ __forceinline__ void load4_f32(const float* p, float* v) {
+  float4 t;
+  if constexpr (STREAM) t = __ldcs(reinterpret_cast<const float4*>(p));
+  else t = *reinterpret_cast<const float4*>(p);
+  v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
+}
+template <bool STREAM>
+__device__ __forceinline__ void load4_f32(const __half* p, float* v) {
+  uint2 t;
+  if constexpr (STREAM) t = __ldcs(reinterpret_cast<const uint2*>(p));
+  else t = *reinterpret_cast<const uint2*>(p);
+  const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&t.x));
+  const float2 b = __half22float2(*reinterpret_cast<const __half2*>(&t.y));
+  v[0] = a.x; v[1] = a.y; v[2] = b.x; v[3] = b.y;
+}
+template <bool STREAM>
+__device__ __forceinline__ void load4_f32(const __nv_bfloat16* p, float* v) {
+  uint2 t;
+  if constexpr (STREAM) t = __ldcs(reinterpret_cast<const uint2*>(p));
+  else t = *reinterpret_cast<const uint2*>(p);
+  const float2 a = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&t.x));
+  const float2 b = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&t.y));
+  v[0] = a.x; v[1] = a.y; v[2] = b.x; v[3] = b.y;
+}
 
 }  // namespace lcrec

@@ -386,22 +386,25 @@ linear_pair_kernel(const __grid_constant__ CUtensorMap map_ahi, const __grid_con
   }
 }
 
-// x (rows, k) fp32 -> group-scaled fp16 pair, one pass: a warp owns a row, each iteration covers one 256-element
-// group (two float4 per lane), group maximum by warp shuffles.  Scales are staged in shared memory and written
-// group-major ([group][row], coalesced over rows) - the layout the fold warps read.
+// x (rows, k) fp32 / fp16 / bf16 -> group-scaled fp16 pair, one pass: a warp owns a row, each iteration covers one
+// 256-element group (two 4-element vectors per lane: float4, or 8 bytes of halves), group maximum by warp shuffles.
+// Every element is converted to fp32 on load (exact for both half formats), so a half input gives the bits the fp32
+// input x.float() gives.  Scales are staged in shared memory and written group-major ([group][row], coalesced over
+// rows) - the layout the fold warps read.
 constexpr int kSplitRowsPerCta = 32;
-__global__ void __launch_bounds__(256) split_groups_kernel(const float* __restrict__ x, int64_t rows, int k, int64_t ldx,
+template <typename T>
+__global__ void __launch_bounds__(256) split_groups_kernel(const T* __restrict__ x, int64_t rows, int k, int64_t ldx,
                                                            __half* __restrict__ hi, __half* __restrict__ lo, int64_t ld_out,
                                                            float* __restrict__ inv_scale, int64_t ld_scale, int n_groups) {
   extern __shared__ float s_scale[];                 // n_groups x 32 rows
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const bool vec_ok = ((ldx & 3) == 0) && ((reinterpret_cast<uintptr_t>(x) & 15) == 0);
+  const bool vec_ok = ((ldx & 3) == 0) && ((reinterpret_cast<uintptr_t>(x) & (4 * sizeof(T) - 1)) == 0);
   for (int64_t blk = blockIdx.x; blk * kSplitRowsPerCta < rows; blk += gridDim.x) {
     const int64_t r0 = blk * kSplitRowsPerCta;
     for (int rr = warp; rr < kSplitRowsPerCta; rr += 8) {
       const int64_t r = r0 + rr;
       if (r >= rows) { for (int g = lane; g < n_groups; g += 32) s_scale[g * 32 + rr] = 1.f; continue; }
-      const float* xr = x + r * ldx;
+      const T* xr = x + r * ldx;
       __half* hr = hi + r * ld_out;
       __half* lr = lo + r * ld_out;
 #pragma unroll 2
@@ -411,11 +414,10 @@ __global__ void __launch_bounds__(256) split_groups_kernel(const float* __restri
         for (int hseg = 0; hseg < 2; ++hseg) {
           const int c = g * kGroup + hseg * 128 + lane * 4;
           if (vec_ok && c + 3 < k) {
-            const float4 t = __ldcs(reinterpret_cast<const float4*>(xr + c));
-            v[4 * hseg] = t.x; v[4 * hseg + 1] = t.y; v[4 * hseg + 2] = t.z; v[4 * hseg + 3] = t.w;
+            load4_f32<true>(xr + c, v + 4 * hseg);
           } else {
 #pragma unroll
-            for (int i = 0; i < 4; ++i) v[4 * hseg + i] = (c + i < k) ? xr[c + i] : 0.f;
+            for (int i = 0; i < 4; ++i) v[4 * hseg + i] = (c + i < k) ? to_f32(xr[c + i]) : 0.f;
           }
         }
         float m = 0.f;
@@ -543,16 +545,27 @@ int launch_argmin_pair(const PairProblem& p, cudaStream_t st) {
   return launch_pair_cfg<64, 3, true>(p, st);
 }
 
-int launch_split_groups(const float* x, int64_t rows, int k, int64_t ldx, __half* hi, __half* lo, int64_t ld_out,
-                        float* inv_scale, int64_t ld_scale, cudaStream_t st) {
+template <typename T>
+static int launch_split_groups_t(const T* x, int64_t rows, int k, int64_t ldx, __half* hi, __half* lo, int64_t ld_out,
+                                 float* inv_scale, int64_t ld_scale, cudaStream_t st) {
   if (rows == 0) return LCREC_OK;
   const int n_groups = (int)ceil_div(ld_out, kGroup);
   const size_t smem = sizeof(float) * 32 * n_groups;
   if (smem > 48 * 1024) { set_error("split_groups: k = %d too wide", k); return LCREC_ERR_UNSUPPORTED; }
   const int64_t blocks = std::min<int64_t>(ceil_div(rows, kSplitRowsPerCta), (int64_t)num_sms() * 8);
-  split_groups_kernel<<<(unsigned)blocks, 256, smem, st>>>(x, rows, k, ldx, hi, lo, ld_out, inv_scale, ld_scale, n_groups);
+  split_groups_kernel<T><<<(unsigned)blocks, 256, smem, st>>>(x, rows, k, ldx, hi, lo, ld_out, inv_scale, ld_scale, n_groups);
   LC_LAUNCH_CHECK("split_groups_kernel");
   return LCREC_OK;
+}
+
+int launch_split_groups(const void* x, int dtype, int64_t rows, int k, int64_t ldx, __half* hi, __half* lo, int64_t ld_out,
+                        float* inv_scale, int64_t ld_scale, cudaStream_t st) {
+  switch (dtype) {
+    case kDtypeF32: return launch_split_groups_t(static_cast<const float*>(x), rows, k, ldx, hi, lo, ld_out, inv_scale, ld_scale, st);
+    case kDtypeF16: return launch_split_groups_t(static_cast<const __half*>(x), rows, k, ldx, hi, lo, ld_out, inv_scale, ld_scale, st);
+    case kDtypeBF16: return launch_split_groups_t(static_cast<const __nv_bfloat16*>(x), rows, k, ldx, hi, lo, ld_out, inv_scale, ld_scale, st);
+    default: set_error("split_groups: bad argument: dtype %d (0 = fp32, 1 = fp16, 2 = bf16)", dtype); return LCREC_ERR_ARG;
+  }
 }
 
 }  // namespace lcrec

@@ -278,27 +278,29 @@ __global__ void split_tf32_kernel(const float* __restrict__ x, int64_t rows, int
   }
 }
 
-// x (rows, k) fp32 -> per-row power-of-two scale s with max|x s| in [2^14, 2^15), hi = fp16(x s),
+// x (rows, k) fp32 / fp16 / bf16 -> per-row power-of-two scale s with max|x s| in [2^14, 2^15), hi = fp16(x s),
 // lo = fp16(x s - hi) (both padded with zeros to ld_out), inv_scale[row] = 1 / s.  One warp per row, two
-// passes over the row (the second one hits L1/L2).
-__global__ void __launch_bounds__(256) split_f16_rows_kernel(const float* __restrict__ x, int64_t rows, int k, int64_t ldx,
+// passes over the row (the second one hits L1/L2).  Half inputs are converted to fp32 on load (exact).
+template <typename T>
+__global__ void __launch_bounds__(256) split_f16_rows_kernel(const T* __restrict__ x, int64_t rows, int k, int64_t ldx,
                                                              __half* __restrict__ hi, __half* __restrict__ lo, int64_t ld_out,
                                                              float* __restrict__ inv_scale) {
   const int lane = threadIdx.x & 31;
   const int64_t warp0 = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
   const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-  const bool vec_ok = ((ldx & 3) == 0) && ((reinterpret_cast<uintptr_t>(x) & 15) == 0);
+  const bool vec_ok = ((ldx & 3) == 0) && ((reinterpret_cast<uintptr_t>(x) & (4 * sizeof(T) - 1)) == 0);
   for (int64_t r = warp0; r < rows; r += nwarps) {
-    const float* xr = x + r * ldx;
+    const T* xr = x + r * ldx;
     float m = 0.f;
     if (vec_ok) {
       for (int c = lane * 4; c + 3 < k; c += 128) {
-        const float4 t = *reinterpret_cast<const float4*>(xr + c);
-        m = fmaxf(fmaxf(m, fmaxf(fabsf(t.x), fabsf(t.y))), fmaxf(fabsf(t.z), fabsf(t.w)));
+        float t[4];
+        load4_f32<false>(xr + c, t);
+        m = fmaxf(fmaxf(m, fmaxf(fabsf(t[0]), fabsf(t[1]))), fmaxf(fabsf(t[2]), fabsf(t[3])));
       }
-      for (int c = (k & ~3) + lane; c < k; c += 32) m = fmaxf(m, fabsf(xr[c]));
+      for (int c = (k & ~3) + lane; c < k; c += 32) m = fmaxf(m, fabsf(to_f32(xr[c])));
     } else {
-      for (int c = lane; c < k; c += 32) m = fmaxf(m, fabsf(xr[c]));
+      for (int c = lane; c < k; c += 32) m = fmaxf(m, fabsf(to_f32(xr[c])));
     }
     for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
     // exponent-only scale: s = 2^(14 - floor(log2 m)); m == 0, inf or nan -> s = 1
@@ -315,11 +317,10 @@ __global__ void __launch_bounds__(256) split_f16_rows_kernel(const float* __rest
     for (int c = lane * 4; c < ld_out; c += 128) {
       float v[4];
       if (vec_ok && c + 3 < k) {
-        const float4 t = *reinterpret_cast<const float4*>(xr + c);
-        v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
+        load4_f32<false>(xr + c, v);
       } else {
 #pragma unroll
-        for (int i = 0; i < 4; ++i) v[i] = (c + i < k) ? xr[c + i] : 0.f;
+        for (int i = 0; i < 4; ++i) v[i] = (c + i < k) ? to_f32(xr[c + i]) : 0.f;
       }
       __half h[4], l[4];
 #pragma unroll
@@ -427,13 +428,30 @@ int launch_linear(const LinearProblem& p, cudaStream_t st) {
   return launch_cfg<32, 32, 4>(p, st);
 }
 
-int launch_split_f16(const float* x, int64_t rows, int k, int64_t ldx, __half* hi, __half* lo, int64_t ld_out,
-                     float* inv_scale, cudaStream_t st) {
+template <typename T>
+static int launch_split_f16_t(const T* x, int64_t rows, int k, int64_t ldx, __half* hi, __half* lo, int64_t ld_out,
+                              float* inv_scale, cudaStream_t st) {
   if (rows == 0) return LCREC_OK;
   const int64_t blocks = std::min<int64_t>(ceil_div(rows, 8), (int64_t)num_sms() * 16);
-  split_f16_rows_kernel<<<(unsigned)blocks, 256, 0, st>>>(x, rows, k, ldx, hi, lo, ld_out, inv_scale);
+  split_f16_rows_kernel<T><<<(unsigned)blocks, 256, 0, st>>>(x, rows, k, ldx, hi, lo, ld_out, inv_scale);
   LC_LAUNCH_CHECK("split_f16_rows_kernel");
   return LCREC_OK;
+}
+
+int launch_split_f16(const float* x, int64_t rows, int k, int64_t ldx, __half* hi, __half* lo, int64_t ld_out,
+                     float* inv_scale, cudaStream_t st) {
+  return launch_split_f16_t(x, rows, k, ldx, hi, lo, ld_out, inv_scale, st);
+}
+
+// the same for x of element type `dtype` (kDtypeF32 / kDtypeF16 / kDtypeBF16)
+static int launch_split_f16_ex(const void* x, int dtype, int64_t rows, int k, int64_t ldx, __half* hi, __half* lo, int64_t ld_out,
+                               float* inv_scale, cudaStream_t st) {
+  switch (dtype) {
+    case kDtypeF32: return launch_split_f16_t(static_cast<const float*>(x), rows, k, ldx, hi, lo, ld_out, inv_scale, st);
+    case kDtypeF16: return launch_split_f16_t(static_cast<const __half*>(x), rows, k, ldx, hi, lo, ld_out, inv_scale, st);
+    case kDtypeBF16: return launch_split_f16_t(static_cast<const __nv_bfloat16*>(x), rows, k, ldx, hi, lo, ld_out, inv_scale, st);
+    default: set_error("split_f16_rows: bad argument: dtype %d (0 = fp32, 1 = fp16, 2 = bf16)", dtype); return LCREC_ERR_ARG;
+  }
 }
 
 int launch_split(const float* x, int64_t rows, int k, int64_t ldx, float* hi, float* lo, int64_t ld_out,
@@ -585,7 +603,7 @@ extern "C" int64_t lcrec_mlp_workspace_bytes(const lcrec_mlp_t* m, int64_t n_row
 // f16 x3 engine.  Wide layers (n_out a multiple of 256) run on the CTA-pair kernel with group-scaled operands and
 // hand the next wide layer its fp16 hi/lo operand straight from the epilogue; the narrow tail layers use the
 // single-CTA kernel with per-row scales (fp32 activation + split_f16_rows pass in between).
-static int mlp_forward_f16(lcrec_mlp_t* m, const float* x, int64_t n_rows, float* y, float* const* acts, void* workspace,
+static int mlp_forward_f16(lcrec_mlp_t* m, const void* x, int dtype, int64_t n_rows, float* y, float* const* acts, void* workspace,
                            int64_t workspace_bytes, cudaStream_t st) {
   Arena ar(workspace, workspace_bytes);
   const int64_t ld0 = ld8(m->dims[0]);
@@ -601,8 +619,8 @@ static int mlp_forward_f16(lcrec_mlp_t* m, const float* x, int64_t n_rows, float
   if (!ar.ok()) { set_error("mlp_forward: workspace too small (%lld bytes given, %lld needed)", (long long)workspace_bytes, (long long)lcrec_mlp_workspace_bytes(m, n_rows)); return LCREC_ERR_NOMEM; }
   const bool allow_pair = !(m->variant & 16);
   auto pair_ok = [&](int l) { return allow_pair && l < m->n_layers && linear_pair_supported(m->dims[l], m->dims[l + 1], kPairGroup); };
-  // current activation: fp32 (cur, ldc) or group-scaled fp16 (grp)
-  const float* cur = x; int64_t ldc = m->dims[0];
+  // current activation: (cur, ldc) of element type cur_dtype (the input's for layer 0, fp32 after it) or group-scaled fp16 (grp)
+  const void* cur = x; int cur_dtype = dtype; int64_t ldc = m->dims[0];
   SplitOperand grp{}; bool grouped = false; int next_set = 0;
   for (int l = 0; l < m->n_layers; ++l) {
     const bool last = (l == m->n_layers - 1);
@@ -615,7 +633,7 @@ static int mlp_forward_f16(lcrec_mlp_t* m, const float* x, int64_t n_rows, float
         __half* lo = l == 0 ? in_lo : set_lo[next_set];
         float* sc = l == 0 ? in_scale : set_scale[next_set];
         if (l != 0) next_set ^= 1;
-        LC_TRY(launch_split_groups(cur, n_rows, k, ldc, hi, lo, ld8(k), sc, n_rows, st));
+        LC_TRY(launch_split_groups(cur, cur_dtype, n_rows, k, ldc, hi, lo, ld8(k), sc, n_rows, st));
         grp.hi = hi; grp.lo = lo; grp.ld = ld8(k); grp.inv_scale = sc; grp.ld_scale = n_rows; grp.group = kPairGroup;
         grouped = true;
       }
@@ -638,14 +656,14 @@ static int mlp_forward_f16(lcrec_mlp_t* m, const float* x, int64_t n_rows, float
         grp.hi = p.o_hi; grp.lo = p.o_lo; grp.ld = p.ldo; grp.inv_scale = p.o_inv_scale; grp.ld_scale = n_rows; grp.group = kPairGroup;
         next_set ^= 1;
       } else {
-        grouped = false; cur = p.y; ldc = p.ldy;
+        grouped = false; cur = p.y; cur_dtype = kDtypeF32; ldc = p.ldy;
       }
       continue;
     }
     // single-CTA kernel, per-row scales
     {
       ProfScope prof(l == 0 ? 0 : 17, st);
-      LC_TRY(launch_split_f16(cur, n_rows, k, ldc, l == 0 ? in_hi : set_hi[0], l == 0 ? in_lo : set_lo[0], ld8(k), rscale, st));
+      LC_TRY(launch_split_f16_ex(cur, cur_dtype, n_rows, k, ldc, l == 0 ? in_hi : set_hi[0], l == 0 ? in_lo : set_lo[0], ld8(k), rscale, st));
     }
     LinearProblem p{};
     p.f16 = true; p.row_scale = rscale; p.col_scale = m->h_scale[l];
@@ -661,7 +679,7 @@ static int mlp_forward_f16(lcrec_mlp_t* m, const float* x, int64_t n_rows, float
       return LCREC_ERR_UNSUPPORTED;
     }
     { ProfScope prof(1 + std::min(l, 15), st); LC_TRY(launch_linear(p, st)); }
-    cur = out; ldc = ldo;
+    cur = out; cur_dtype = kDtypeF32; ldc = ldo;
   }
   if (acts && acts[m->n_layers - 1] && acts[m->n_layers - 1] != y)
     LC_CUDA(cudaMemcpyAsync(acts[m->n_layers - 1], y, sizeof(float) * n_rows * m->dims[m->n_layers], cudaMemcpyDeviceToDevice, st));
@@ -670,11 +688,22 @@ static int mlp_forward_f16(lcrec_mlp_t* m, const float* x, int64_t n_rows, float
 
 extern "C" int lcrec_mlp_forward(lcrec_mlp_t* m, const float* x, int64_t n_rows, float* y, float* const* acts,
                                  void* workspace, int64_t workspace_bytes, void* stream) {
+  return lcrec_mlp_forward_ex(m, x, kDtypeF32, n_rows, y, acts, workspace, workspace_bytes, stream);
+}
+
+extern "C" int lcrec_mlp_forward_ex(lcrec_mlp_t* m, const void* x_in, int dtype, int64_t n_rows, float* y, float* const* acts,
+                                    void* workspace, int64_t workspace_bytes, void* stream) {
+  LC_ARG(dtype_ok(dtype));
   LC_ARG(m != nullptr && n_rows >= 0);
   if (n_rows == 0) return LCREC_OK;
-  LC_ARG(x != nullptr && y != nullptr);
+  LC_ARG(x_in != nullptr && y != nullptr);
   cudaStream_t st = (cudaStream_t)stream;
-  if (m->engine == 1) return mlp_forward_f16(m, x, n_rows, y, acts, workspace, workspace_bytes, st);
+  if (m->engine == 1) return mlp_forward_f16(m, x_in, dtype, n_rows, y, acts, workspace, workspace_bytes, st);
+  if (dtype != kDtypeF32) {
+    set_error("mlp_forward: engine 0 (tf32 x3) takes fp32 input only (dtype %d); half-precision input needs engine 1 (f16 x3)", dtype);
+    return LCREC_ERR_UNSUPPORTED;
+  }
+  const float* x = static_cast<const float*>(x_in);
   Arena ar(workspace, workspace_bytes);
   const int64_t ld0 = ld4(m->dims[0]);
   float* in_hi = ar.take<float>(n_rows * ld0);
@@ -736,7 +765,7 @@ extern "C" int lcrec_linear_forward(const float* x, int64_t n_rows, int k_in, co
     float* cs = ar.take<float>(n_out);
     float* as = ar.take<float>(n_rows * ceil_div(ldk, kPairGroup));
     if (!ar.ok()) { set_error("linear_forward: workspace too small"); return LCREC_ERR_NOMEM; }
-    LC_TRY(launch_split_groups(x, n_rows, k_in, k_in, a_hi, a_lo, ldk, as, n_rows, st));
+    LC_TRY(launch_split_groups(x, kDtypeF32, n_rows, k_in, k_in, a_hi, a_lo, ldk, as, n_rows, st));
     LC_TRY(launch_split_f16(w, n_out, k_in, k_in, w_hi, w_lo, ldk, cs, st));
     PairProblem q{};
     q.a.hi = a_hi; q.a.lo = a_lo; q.a.ld = ldk; q.a.inv_scale = as; q.a.ld_scale = n_rows; q.a.group = kPairGroup;

@@ -79,6 +79,7 @@ class CudaBackend:
         self.iters = int(model.rq.vq_layers[-1].sk_iters)
 
     def pass0(self, x_local: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Codes + last-level residuals of this rank's shard; an fp16 / bf16 shard is read as it is (Indexer.pass0)."""
         n = x_local.shape[0]
         if n == 0:
             dev = self.cbs[0].device

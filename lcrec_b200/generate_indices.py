@@ -53,12 +53,14 @@ def generate_codes(model: RQVAE, data, max_rounds: int = 20, chunk_rows: int = 1
     """Collision-resolved codes for every row of ``data``.
 
     ``data``: CUDA float tensor (device-resident path) or CPU tensor / ndarray / EmbDataset (host
-    path: embeddings are streamed to the device in chunks).  Returns (codes int64 CPU tensor, stats).
+    path: embeddings are streamed to the device in chunks).  fp16 / bf16 embeddings are indexed as they are
+    (an fp16 ndarray or ``.npy`` is not converted; the codes equal those of its fp32 upcast); other ndarray
+    dtypes become an fp32 copy.  Returns (codes int64 CPU tensor, stats).
     """
     if isinstance(data, EmbDataset):
         data = data.embeddings
     if isinstance(data, np.ndarray):
-        data = torch.from_numpy(np.ascontiguousarray(data, dtype=np.float32))
+        data = torch.from_numpy(np.ascontiguousarray(data, dtype=np.float16 if data.dtype == np.float16 else np.float32))
     n = int(data.shape[0])
     ix = indexer or build_indexer(model, max(n, 1), min(chunk_rows, max(n, 1)))
     if data.is_cuda:

@@ -569,7 +569,8 @@ def codebook_usage(cluster_size: torch.Tensor, epsilon: float, reset_threshold: 
 
 
 # --------------------------------------------------------------------------- embedding producer hand-off
-_POOL_DTYPES = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}
+# element type codes of the C ABI's `dtype` arguments: the hidden states of the pool, the embeddings of the _ex indexer entries
+DTYPE_CODES = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}
 
 
 def masked_mean_pool(last_hidden_state: torch.Tensor, attention_mask: torch.Tensor, out: Optional[torch.Tensor] = None,
@@ -579,7 +580,7 @@ def masked_mean_pool(last_hidden_state: torch.Tensor, attention_mask: torch.Tens
     ``accumulate`` adds to ``out``; ``divide_by`` > 0 divides the result (mean over text fields, :96)."""
     _need_cuda(last_hidden_state, attention_mask, out)
     lib = _lib.load()
-    if last_hidden_state.dtype not in _POOL_DTYPES:
+    if last_hidden_state.dtype not in DTYPE_CODES:
         raise RuntimeError(f"masked_mean_pool: unsupported hidden dtype {last_hidden_state.dtype}")
     h = last_hidden_state.detach().contiguous()
     b, t, d = h.shape
@@ -595,7 +596,7 @@ def masked_mean_pool(last_hidden_state: torch.Tensor, attention_mask: torch.Tens
     stride = out.stride(0) if b > 1 else max(d, out.stride(0))
     ws = _ws(lib.lcrec_masked_mean_pool_workspace_bytes(b, t, d), h.device)
     with torch.cuda.device(h.device):
-        _lib.check(lib.lcrec_masked_mean_pool(_p(h), _POOL_DTYPES[h.dtype], _p(m), b, t, d, _p(out), stride,
+        _lib.check(lib.lcrec_masked_mean_pool(_p(h), DTYPE_CODES[h.dtype], _p(m), b, t, d, _p(out), stride,
                                               int(accumulate), float(divide_by), _p(ws), ws.numel(), _stream(h)))
     return out
 
@@ -788,6 +789,17 @@ def index_json_bytes(codes: torch.Tensor) -> bytes:
 
 
 # --------------------------------------------------------------------------- whole generation
+_HALF = (torch.float16, torch.bfloat16)
+
+
+def _embeddings(x: torch.Tensor) -> Tuple[torch.Tensor, Optional[int]]:
+    """(tensor, dtype code) for the indexer entries: fp16 / bf16 embeddings stay as they are (contiguous; the kernels read
+    them natively, code 1 / 2); every other dtype becomes an fp32 copy as before (code None: the fp32 entry)."""
+    if x.dtype in _HALF:
+        return x.detach().contiguous(), DTYPE_CODES[x.dtype]
+    return _f32c(x), None
+
+
 class Indexer:
     """generate_indices.py:85-128 on the device (PASS 0 + collision rounds)."""
 
@@ -813,27 +825,38 @@ class Indexer:
         return {k: int(raw[i]) for i, k in enumerate(keys)}
 
     def run_device(self, x: torch.Tensor, max_rounds: int = 20) -> Tuple[torch.Tensor, dict]:
+        """x: CUDA (n, in_dim) embeddings.  fp16 / bf16 are read as they are (no fp32 copy); the codes and stats are
+        those of the fp32 run on ``x.float()``, bit for bit."""
         _need_cuda(x)
-        x2 = _f32c(x)
+        x2, code = _embeddings(x)
         n = x2.shape[0]
         codes = torch.empty((n, self.L), dtype=torch.int64, device=x2.device)
         stats = (C.c_int64 * 8)()
         with torch.cuda.device(x2.device):
-            _lib.check(self.lib.lcrec_indexer_run_device(self.handle, _p(x2), n, int(max_rounds), _p(codes), stats,
-                                                         _stream(x2)))
+            if code is None:
+                _lib.check(self.lib.lcrec_indexer_run_device(self.handle, _p(x2), n, int(max_rounds), _p(codes), stats,
+                                                             _stream(x2)))
+            else:
+                _lib.check(self.lib.lcrec_indexer_run_device_ex(self.handle, _p(x2), code, n, int(max_rounds), _p(codes),
+                                                                stats, _stream(x2)))
         return codes, self._stats(stats)
 
     def run_host(self, x_host, codes_host=None, max_rounds: int = 20):
-        """x_host: CPU float32 tensor / ndarray (n, in_dim) (pinned or pageable); returns CPU int64 codes."""
+        """x_host: CPU float32 / float16 / bfloat16 tensor or ndarray (n, in_dim), contiguous (pinned or pageable); half
+        precision is copied to the device as it is (half the bytes).  Returns CPU int64 codes."""
         xt = torch.as_tensor(x_host)
-        assert not xt.is_cuda and xt.dtype == torch.float32 and xt.is_contiguous()
+        assert not xt.is_cuda and xt.dtype in (torch.float32,) + _HALF and xt.is_contiguous()
         n = xt.shape[0]
         out = torch.empty((n, self.L), dtype=torch.int64) if codes_host is None else codes_host
         stats = (C.c_int64 * 8)()
         with torch.cuda.device(self.device):
             st = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-            _lib.check(self.lib.lcrec_indexer_run_host(self.handle, C.c_void_p(xt.data_ptr()), n, int(max_rounds),
-                                                       C.c_void_p(out.data_ptr()), stats, st))
+            if xt.dtype == torch.float32:
+                _lib.check(self.lib.lcrec_indexer_run_host(self.handle, C.c_void_p(xt.data_ptr()), n, int(max_rounds),
+                                                           C.c_void_p(out.data_ptr()), stats, st))
+            else:
+                _lib.check(self.lib.lcrec_indexer_run_host_ex(self.handle, C.c_void_p(xt.data_ptr()), DTYPE_CODES[xt.dtype], n,
+                                                              int(max_rounds), C.c_void_p(out.data_ptr()), stats, st))
         return out, self._stats(stats)
 
     def resolve_device(self, codes: torch.Tensor, resid: torch.Tensor, max_rounds: int = 20) -> dict:
@@ -847,9 +870,13 @@ class Indexer:
         return self._stats(stats)
 
     def pass0(self, x: torch.Tensor, row_offset: int = 0) -> None:
-        x2 = _f32c(x)
+        x2, code = _embeddings(x)
         with torch.cuda.device(x2.device):
-            _lib.check(self.lib.lcrec_indexer_pass0(self.handle, _p(x2), x2.shape[0], int(row_offset), _stream(x2)))
+            if code is None:
+                _lib.check(self.lib.lcrec_indexer_pass0(self.handle, _p(x2), x2.shape[0], int(row_offset), _stream(x2)))
+            else:
+                _lib.check(self.lib.lcrec_indexer_pass0_ex(self.handle, _p(x2), code, x2.shape[0], int(row_offset),
+                                                           _stream(x2)))
 
     def round(self, n: int) -> dict:
         counts = (C.c_int64 * 4)()

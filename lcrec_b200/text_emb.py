@@ -7,6 +7,10 @@ happens to ``outputs.last_hidden_state`` is ours: the masked mean pool (:91-92) 
 ``Indexer.run`` / ``lcrec_indexer_run_device`` reads - instead of a Python list of CPU tensors, a ``torch.cat`` and an
 ``.npy`` round trip.  The ``.npy`` file of the reference (``<root>/<dataset>.emb-<plm_name>-td.npy``, :104-105) is still
 written unless ``save=False``; the device matrix is returned.
+
+``dtype=torch.float16`` / ``torch.bfloat16`` keeps the matrix in half precision (half the memory, and the indexer reads it
+without an fp32 copy): each batch is pooled into an fp32 scratch of ``batch_size`` rows as above and rounded once into its
+rows, so the matrix equals the fp32 one ``.to(dtype)``.  An fp16 matrix is saved as an fp16 ``.npy``; numpy has no bf16.
 """
 from __future__ import annotations
 
@@ -20,9 +24,16 @@ from . import ops
 
 
 @torch.no_grad()
-def generate_item_embedding(args, item_text_list, tokenizer, model, word_drop_ratio=-1, batch_size=1, save=True):
-    """args: .root, .dataset, .plm_name, .max_sent_len, .device (a CUDA device).  Returns the (N, hidden) fp32 device matrix.
-    ``batch_size`` 1 is the reference's hard-coded value (:61); larger batches pool several items per launch."""
+def generate_item_embedding(args, item_text_list, tokenizer, model, word_drop_ratio=-1, batch_size=1, save=True,
+                            dtype=torch.float32):
+    """args: .root, .dataset, .plm_name, .max_sent_len, .device (a CUDA device).  Returns the (N, hidden) device matrix of
+    ``dtype`` (fp32, fp16 or bf16).  ``batch_size`` 1 is the reference's hard-coded value (:61); larger batches pool several
+    items per launch."""
+    if dtype not in (torch.float32, torch.float16, torch.bfloat16):
+        raise ValueError(f"generate_item_embedding: dtype must be float32, float16 or bfloat16, not {dtype}")
+    if save and dtype == torch.bfloat16:
+        raise ValueError("generate_item_embedding: numpy has no bfloat16, so a bf16 matrix cannot be saved as .npy "
+                         "(use save=False, or dtype=torch.float16)")
     print("Generate Text Embedding: ")
     print(" Dataset: ", args.dataset)
     items, texts = zip(*item_text_list)
@@ -32,7 +43,7 @@ def generate_item_embedding(args, item_text_list, tokenizer, model, word_drop_ra
     for text in order_texts:
         assert text != [0]
 
-    embeddings = None
+    embeddings = scratch = None
     start = 0
     while start < len(order_texts):
         if (start + 1) % 100 == 0:
@@ -51,9 +62,14 @@ def generate_item_embedding(args, item_text_list, tokenizer, model, word_drop_ra
             outputs = model(input_ids=enc.input_ids, attention_mask=enc.attention_mask)
             h = outputs.last_hidden_state
             if embeddings is None:
-                embeddings = torch.empty((len(order_texts), h.shape[-1]), dtype=torch.float32, device=h.device)
-            ops.masked_mean_pool(h, enc["attention_mask"], out=embeddings[start: start + len(batch)], accumulate=f > 0,
+                embeddings = torch.empty((len(order_texts), h.shape[-1]), dtype=dtype, device=h.device)
+                if dtype != torch.float32:
+                    scratch = torch.empty((batch_size, h.shape[-1]), dtype=torch.float32, device=h.device)
+            rows = embeddings[start: start + len(batch)] if scratch is None else scratch[: len(batch)]
+            ops.masked_mean_pool(h, enc["attention_mask"], out=rows, accumulate=f > 0,
                                  divide_by=float(len(fields)) if f == len(fields) - 1 else 0.0)
+        if scratch is not None:
+            embeddings[start: start + len(batch)].copy_(scratch[: len(batch)])      # one rounding to the half format
         start += batch_size
     print("Embeddings shape: ", tuple(embeddings.shape))
     if save:
