@@ -48,6 +48,12 @@ constexpr int kPairGroup = 256;
 int launch_split_groups(const void* x, int dtype, int64_t rows, int k, int64_t ldx, __half* hi, __half* lo, int64_t ld_out,
                         float* inv_scale, int64_t ld_scale, cudaStream_t st);
 
+// ReLU of the GEMM epilogues: 0 for finite negative values only.  NaN passes like torch.relu; -inf passes too, because
+// with finite operands it only comes from an overflow of the fp32 accumulator (which on the f16 x3 engine carries the
+// channel scale 2^15 / max|w_c|), and a ReLU of it would turn an out-of-range result into a finite 0.  Unlike torch.relu
+// it also keeps a truly -inf pre-activation (an input row holding inf); that row is non-finite either way.
+__device__ __forceinline__ float relu_keep_nonfinite(float t) { return (t < 0.f && t > -INFINITY) ? 0.f : t; }
+
 // Input loads of the operand splits.  Both half formats convert to fp32 exactly, so everything after the load is the
 // arithmetic of the fp32 input.
 __device__ __forceinline__ float to_f32(float v) { return v; }

@@ -296,8 +296,9 @@ linear_pair_kernel(const __grid_constant__ CUtensorMap map_ahi, const __grid_con
         float4 bv = make_float4(0.f, 0.f, 0.f, 0.f);
         if (args.bias) bv = __ldg(reinterpret_cast<const float4*>(args.bias + col_base + j));
         float t0 = acc[j] * cs.x + bv.x, t1 = acc[j + 1] * cs.y + bv.y, t2 = acc[j + 2] * cs.z + bv.z, t3 = acc[j + 3] * cs.w + bv.w;
-        // ReLU that lets NaN through like torch.relu (fmaxf(NaN, 0) would be 0 and hide a diverged run from trainer.py:93-95)
-        if (args.relu) { t0 = t0 < 0.f ? 0.f : t0; t1 = t1 < 0.f ? 0.f : t1; t2 = t2 < 0.f ? 0.f : t2; t3 = t3 < 0.f ? 0.f : t3; }
+        // ReLU that lets NaN through like torch.relu (fmaxf(NaN, 0) would be 0 and hide a diverged run from trainer.py:93-95),
+        // and an accumulator overflow to -inf (linear.cuh)
+        if (args.relu) { t0 = relu_keep_nonfinite(t0); t1 = relu_keep_nonfinite(t1); t2 = relu_keep_nonfinite(t2); t3 = relu_keep_nonfinite(t3); }
         acc[j] = t0; acc[j + 1] = t1; acc[j + 2] = t2; acc[j + 3] = t3;
         amax = fmaxf(fmaxf(amax, fmaxf(fabsf(t0), fabsf(t1))), fmaxf(fabsf(t2), fabsf(t3)));
       }
@@ -339,7 +340,7 @@ linear_pair_kernel(const __grid_constant__ CUtensorMap map_ahi, const __grid_con
         float s = 1.f, is = 1.f;
         if (amax > 0.f && amax < INFINITY) {
           const int e = (int)((__float_as_uint(amax) >> 23) & 0xffu) - 127;      // floor(log2 amax) (normal numbers)
-          const int sh = min(max(14 - e, -100), 100);
+          const int sh = min(max(14 - e, -126), 126);
           s = __uint_as_float((uint32_t)(sh + 127) << 23); is = __uint_as_float((uint32_t)(127 - sh) << 23);
         }
         if (row_ok && half == 0) args.o_inv_scale[(int64_t)tile_n * args.ld_oscale + row] = is;
@@ -429,7 +430,7 @@ __global__ void __launch_bounds__(256) split_groups_kernel(const T* __restrict__
         if (m > 0.f && m < INFINITY) {
           int e;
           frexpf(m, &e);                               // floor(log2 m) = e - 1 (also for subnormal m)
-          const int sh = min(max(15 - e, -100), 100);
+          const int sh = min(max(15 - e, -126), 126);
           s = ldexpf(1.f, sh); is = ldexpf(1.f, -sh);
         }
         if (lane == 0) s_scale[g * 32 + rr] = is;

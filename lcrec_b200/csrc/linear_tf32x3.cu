@@ -224,7 +224,7 @@ linear_split3_kernel(const __grid_constant__ CUtensorMap map_ahi, const __grid_c
           float t = acc[j + i];
           if constexpr (F16) { if (col + i < args.n_out) t = (t * rscale) * (args.col_scale ? __ldg(args.col_scale + col + i) : 1.f); }
           if (args.bias != nullptr && col + i < args.n_out) t += __ldg(args.bias + col + i);
-          if (args.relu) t = t < 0.f ? 0.f : t;            // NaN passes, like torch.relu
+          if (args.relu) t = relu_keep_nonfinite(t);       // NaN passes, like torch.relu; so does an overflow to -inf
           v[i] = t;
           hi[i] = to_tf32(t);
           lo[i] = to_tf32(t - hi[i]);
@@ -308,7 +308,7 @@ __global__ void __launch_bounds__(256) split_f16_rows_kernel(const T* __restrict
     if (m > 0.f && m < INFINITY) {
       int e;
       frexpf(m, &e);                 // m = f * 2^e, f in [0.5, 1)  ->  floor(log2 m) = e - 1
-      const int sh = min(max(15 - e, -100), 100);
+      const int sh = min(max(15 - e, -126), 126);
       s = ldexpf(1.f, sh); is = ldexpf(1.f, -sh);
     }
     if (lane == 0) inv_scale[r] = is;

@@ -318,7 +318,7 @@ __global__ void __launch_bounds__(256) rq_tc_prepare_kernel(const RqTcPrep a) {
         if (m > 0.f && m < INFINITY) {
           int e;
           frexpf(m, &e);
-          const int sh = min(max(15 - e, -100), 100);
+          const int sh = min(max(15 - e, -126), 126);
           s = ldexpf(1.f, sh); is = ldexpf(1.f, -sh);
         }
         if (lane == 0) a.inv_scale[(int64_t)(g0 >> 8) * a.ld_scale + i] = is;
@@ -394,7 +394,7 @@ __global__ void __launch_bounds__(256) rq_tc_prepare_small_kernel(const RqTcPrep
       if (m > 0.f && m < INFINITY) {
         int e;
         frexpf(m, &e);
-        const int sh = min(max(15 - e, -100), 100);
+        const int sh = min(max(15 - e, -126), 126);
         s = ldexpf(1.f, sh); is = ldexpf(1.f, -sh);
       }
       a.inv_scale[i] = is;                         // D <= 64: a single scale group
