@@ -411,6 +411,21 @@ int lcrec_ema_update(const float* latent, const int64_t* indices, int64_t n, int
                      void* stream);
 int lcrec_codebook_usage(const float* cluster_size, int n_codes, double epsilon, double reset_threshold,
                          int64_t* used_codes, uint8_t* unused_mask, void* stream);
+/* Data-parallel EMA step: the rows of the global batch are split over `world` ranks in ShardPlan blocks (rank r holds
+ * n_global / world rows, plus one if r < n_global % world; this rank's block is latent (n_local, e_dim), indices
+ * (n_local,)).  Every rank publishes its block into its symmetric buffer, gathers all blocks in rank order into
+ * gathered_latent / gathered_indices (capacity world * rows_per_rank rows each) and runs the lcrec_ema_update kernel on
+ * them with n = n_global: cluster_size, ema_w and codebook end bit-identical to lcrec_ema_update on the concatenated
+ * batch, on every rank.  Three launches on `stream`, no host synchronisation.  peers_dev: device array of `world`
+ * pointers to the ranks' symmetric buffers (lcrec_ema_dist_symmetric_bytes(rows_per_rank, e_dim) each, zeroed once,
+ * peer-mapped); rows_per_rank and e_dim are fixed for a buffer.  epoch = calls made on these buffers so far (0, 1, 2, ...).
+ * flags (1 int32, device, zeroed by the first launch): bit 0 (1) a peer did not arrive, bit 1 (2) a peer published a row count other than
+ * its ShardPlan share.  Collective: every rank calls it, n_local = 0 included.  n_global < 2^31. */
+int64_t lcrec_ema_dist_symmetric_bytes(int64_t rows_per_rank, int e_dim);     /* -1 if rows_per_rank < 1 or e_dim < 1 */
+int lcrec_ema_update_dist(const float* latent, const int64_t* indices, int64_t n_local, int64_t n_global, int n_codes,
+                          int e_dim, double ema_decay, double epsilon, float* cluster_size, float* ema_w, float* codebook,
+                          float* gathered_latent, int64_t* gathered_indices, int32_t* flags, void* const* peers_dev,
+                          int world, int rank, int64_t rows_per_rank, uint64_t epoch, void* stream);
 /* ---- f4: embedding producer hand-off (data_process/amazon_text_emb.py:91-96) -----------------
  * Masked mean pool of a PLM's last hidden state: pooled[b] = sum_t mask[b][t] * hidden[b][t][:] / sum_t mask[b][t]
  * (hidden (n_seq, seq_len, hidden_dim) of dtype 0 = fp32, 1 = fp16, 2 = bf16, row-major; mask (n_seq, seq_len) int64 as

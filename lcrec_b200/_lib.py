@@ -86,6 +86,9 @@ SIGNATURES = {
     "lcrec_indexer_set_speculative": (C.c_int, [C.c_int]),
     "lcrec_ema_update": (C.c_int, [vp, vp, i64, C.c_int, C.c_int, f64, f64, vp, vp, vp, vp]),
     "lcrec_codebook_usage": (C.c_int, [vp, C.c_int, f64, f64, vp, vp, vp]),
+    "lcrec_ema_dist_symmetric_bytes": (i64, [i64, C.c_int]),
+    "lcrec_ema_update_dist": (C.c_int, [vp, vp, i64, i64, C.c_int, C.c_int, f64, f64, vp, vp, vp, vp, vp, vp, vp, C.c_int,
+                                        C.c_int, i64, C.c_uint64, vp]),
     "lcrec_masked_mean_pool_workspace_bytes": (i64, [i64, i64, C.c_int]),
     "lcrec_masked_mean_pool": (C.c_int, [vp, C.c_int, vp, i64, i64, C.c_int, vp, i64, C.c_int, f64, vp, i64, vp]),
     "lcrec_kmeans_workspace_bytes": (i64, [i64, C.c_int, C.c_int]),

@@ -353,3 +353,81 @@ class DistributedSinkhorn:
                                                           _p(flags), _p(self.peers), self.world, self.rank, C.c_uint64(epoch),
                                                           _p(ws), ws.numel(), _stream(d)))
         return q, arg, flags
+
+
+# ----------------------------------------------------------------------------------------------------------------
+# Data-parallel form of the EMA codebook step of index_improve (one step over the global batch, rows split over the ranks)
+class DistributedEma:
+    """The EMA step of index_improve's VectorQuantizer (``lcrec_ema_update``) for a batch whose rows are split over the
+    ranks of ``group`` in ``ShardPlan`` blocks.  Each call gathers every rank's (latent, indices) block through peer memory
+    (symmetric buffers, ``lcrec_ema_update_dist``) and runs the single-device kernel on the concatenated batch, so the
+    buffers end bit-identical to the single-device step on the global batch, on every rank.  One instance serves every
+    level of a model: ``rows_per_rank`` (the largest block, ``ShardPlan(batch_size, world).max_count``) and ``e_dim`` fix
+    the buffer layout; the number of codes and the rows of a call may vary.  Collective: every rank calls ``update``."""
+
+    def __init__(self, rows_per_rank: int, e_dim: int, device, group=None):
+        import torch.distributed._symmetric_memory as symm
+        from . import _lib
+        self.lib = _lib.load()
+        self.group = group if group is not None else dist.group.WORLD
+        self.rows_per_rank, self.e_dim = int(rows_per_rank), int(e_dim)
+        self.device = torch.device(device)
+        nbytes = int(self.lib.lcrec_ema_dist_symmetric_bytes(self.rows_per_rank, self.e_dim))
+        if nbytes <= 0:
+            raise ValueError(f"DistributedEma: rows_per_rank {rows_per_rank} and e_dim {e_dim} must be >= 1")
+        self.buf = symm.empty(nbytes, dtype=torch.uint8, device=self.device)
+        self.buf.zero_()
+        self.hdl = symm.rendezvous(self.buf, self.group)
+        self.world, self.rank = int(self.hdl.world_size), int(self.hdl.rank)
+        self.peers = torch.tensor([int(p) for p in self.hdl.buffer_ptrs], dtype=torch.int64, device=self.device)
+        cap = self.world * self.rows_per_rank
+        self.gathered_latent = torch.empty((cap, self.e_dim), dtype=torch.float32, device=self.device)
+        self.gathered_indices = torch.empty((cap,), dtype=torch.int64, device=self.device)
+        self.epoch = 0                          # calls made on the buffers: the publish counters only grow
+        self.n_rows_hint = None                 # the global row count of the current batch, set by a caller that knows it
+        torch.cuda.synchronize(self.device)
+        dist.barrier(group=self.group)          # every buffer is zeroed and mapped before the first kernel polls it
+
+    def update(self, latent_local: torch.Tensor, indices_local: torch.Tensor, n_global, cluster_size: torch.Tensor,
+               ema_w: torch.Tensor, codebook: torch.Tensor, decay: float, eps: float) -> torch.Tensor:
+        """The EMA step in place on (cluster_size, ema_w, codebook); returns the gathered global latent (n_global, e_dim), a
+        view that the next call overwrites.  ``n_global`` None: ``n_rows_hint``, else an all-reduce of the block sizes."""
+        import ctypes as C
+        from . import _lib
+        from .ops import _inplace_f32, _need_cuda, _p, _stream, check_later
+        _need_cuda(latent_local, indices_local, cluster_size, ema_w, codebook)
+        k, d = codebook.shape
+        if d != self.e_dim:
+            raise ValueError(f"DistributedEma: codebook e_dim {d}, buffers laid out for {self.e_dim}")
+        lat = latent_local.detach().reshape(-1, d).to(torch.float32).contiguous()
+        idx = indices_local.detach().reshape(-1).to(torch.int64).contiguous()
+        n = int(lat.shape[0])
+        if idx.shape[0] != n:
+            raise ValueError("DistributedEma: one index per latent row expected")
+        if n_global is None:
+            n_global = self.n_rows_hint
+        if n_global is None:
+            t = torch.tensor([n], dtype=torch.int64, device=self.device)
+            dist.all_reduce(t, group=self.group)
+            n_global = int(t.item())
+        n_global = int(n_global)
+        plan = ShardPlan(n_global, self.world)
+        # decided from the global row count, which every rank shares: an oversized batch raises on every rank
+        if plan.max_count > self.rows_per_rank:
+            raise ValueError(f"DistributedEma: a block of {plan.max_count} rows exceeds rows_per_rank = {self.rows_per_rank}")
+        # a block other than this rank's ShardPlan share would gather rows the peers never published; raise before any
+        # device work (the peers, if their blocks are right, see this rank's absence through the bounded wait's flag)
+        if n != plan.count(self.rank):
+            raise ValueError(f"DistributedEma: rank {self.rank} holds {n} rows, its ShardPlan share of {n_global} is "
+                             f"{plan.count(self.rank)}")
+        _inplace_f32(cluster_size, "cluster_size"); _inplace_f32(ema_w, "ema_w"); _inplace_f32(codebook, "codebook")
+        flags = torch.empty(1, dtype=torch.int32, device=self.device)
+        epoch = self.epoch
+        self.epoch += 1
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.lcrec_ema_update_dist(_p(lat), _p(idx), n, n_global, k, d, float(decay), float(eps),
+                                                      _p(cluster_size), _p(ema_w), _p(codebook), _p(self.gathered_latent),
+                                                      _p(self.gathered_indices), _p(flags), _p(self.peers), self.world,
+                                                      self.rank, self.rows_per_rank, C.c_uint64(epoch), _stream(lat)))
+        check_later("ema_dist", flags)
+        return self.gathered_latent[:n_global]

@@ -2,8 +2,8 @@
 
 The reference's ``index/trainer.py`` is single-device; the parity target is therefore the single-device step on the GLOBAL
 batch.  One process per GPU (``torch.distributed``, NCCL over NVLink), model replicated, every rank reads the same global
-batches (same loader, same shuffle seed) and takes a contiguous row block of each (``ShardPlan``).  Per step, exactly two
-things cross NVLink, as the north star asks:
+batches (same loader, same shuffle seed) and takes a contiguous row block of each (``ShardPlan``).  Per step, these
+things cross NVLink:
 
 * the Sinkhorn level is ONE (global batch x K) problem (``vq.py:77-79``): ``DistributedSinkhorn`` keeps the row steps local
   and all-reduces the column marginals inside the kernel through peer memory (plus one 2-element MAX all-reduce for the
@@ -12,13 +12,17 @@ things cross NVLink, as the north star asks:
   ``all_reduce(SUM)`` over a flat buffer that holds every gradient (encoder + decoder 89.5 MB, codebooks 128 KB) yields the
   gradient of the global-batch loss on every rank - in ~32 MB buckets that start as soon as autograd has produced their
   gradients (decoder first), overlapping the rest of the backward pass; clipping and the optimiser step then run identically everywhere
-  (``lcrec_adam_clip_step``), so the replicas never diverge.
+  (``lcrec_adam_clip_step``), so the replicas never diverge;
+* for index_improve's EMA-codebook model, per level the row block of the latent and its codes: ``DistributedEma`` gathers
+  every rank's block through peer memory and runs the single-device EMA kernel on the global batch, so counts, sums and
+  codebooks are bit-identical to the single-device step and equal on every rank.  A dead-code reset (every
+  ``reset_interval`` steps, decided from the shared counts) is drawn by rank 0 on the gathered latent and broadcast.
 
 Codebook k-means initialisation (first batch, ``vq.py:67-68``) runs on the full global batch on every rank with the same
 numpy seed, after which rank 0's codebooks are broadcast.  BatchNorm in training mode runs SYNCHRONISED: its kernels all-reduce the
 per-channel sums of the forward and of the backward pass over the ranks (global-batch statistics, identical running
-statistics everywhere).  Refused: the EMA-codebook variant of index_improve/ (its in-place per-rank updates would make the
-replicas diverge).  A rank whose row block is empty still joins the Sinkhorn collectives.  Rank 0 writes checkpoints.
+statistics everywhere).  The k-means pass of an EMA model takes no EMA step (the first batch gets one, in the training
+forward).  A rank whose row block is empty still joins the Sinkhorn and EMA collectives.  Rank 0 writes checkpoints.
 """
 from __future__ import annotations
 
@@ -43,21 +47,17 @@ class DataParallelTrainer(Trainer):
         # BatchNorm (what `run.sh --bn False` really trains, main.py:31): the single-device semantics need batch statistics
         # over the GLOBAL batch -> the BN kernels all-reduce their per-channel sums over the group (forward and backward)
         self._bn_modules = [m for m in model.modules() if isinstance(m, torch.nn.modules.batchnorm._BatchNorm)]
-        if any(name.endswith("_ema_cluster_size") for name, _ in model.named_buffers()):
-            # index_improve's EMA codebooks are updated in place from the rows a rank sees (lcrec_ema_update): with sharded
-            # rows the replicas' counts, sums and codebooks would drift apart from step 1, and the dead-code reset draws
-            # from the local RNG and local latents.  Refused like BatchNorm until the counts and sums are all-reduced.
-            raise NotImplementedError("data-parallel training of the EMA-codebook variant (index_improve) needs the per-code "
-                                      "counts and sums reduced over the ranks before smoothing; train it on one device")
         super().__init__(args, model, data_num)
         self._flat = None
         self._flat_params = None
         self._sinkhorn_levels = []
+        self._ema = None
         for p in self.model.parameters():                       # identical replicas whatever the local seed was
             dist.broadcast(p.data, src=dist.get_global_rank(self.group, 0) if self.group is not dist.group.WORLD else 0,
                            group=self.group)
         if self.device.type == "cuda":
             self._hook_distributed_sinkhorn()
+            self._hook_distributed_ema()
 
     # ---- the Sinkhorn level as one global problem
     def _hook_distributed_sinkhorn(self):
@@ -68,6 +68,26 @@ class DataParallelTrainer(Trainer):
                 if getattr(q, "dist_sinkhorn", None) is None:
                     q.dist_sinkhorn = DistributedSinkhorn(q.n_e, self.device, self.group)
                 self._sinkhorn_levels.append(q)
+
+    # ---- index_improve's EMA codebooks: one EMA step over the global batch
+    def _ema_levels(self):
+        rq = getattr(self.model, "rq", None)
+        return [q for q in (rq.vq_layers if rq is not None else []) if hasattr(q, "_ema_cluster_size")]
+
+    def _hook_distributed_ema(self):
+        """One DistributedEma serves every EMA level (the levels run one after the other on the same stream), sized for the
+        largest row block of a batch of args.batch_size rows.  The EMA buffers are broadcast like the parameters."""
+        from .distributed import DistributedEma
+        levels = self._ema_levels()
+        if not levels:
+            return
+        self._ema = DistributedEma(ShardPlan(int(self.args.batch_size), self.world).max_count, levels[0].e_dim, self.device,
+                                   self.group)
+        src = dist.get_global_rank(self.group, 0) if self.group is not dist.group.WORLD else 0
+        for q in levels:
+            q.dist_ema = self._ema
+            for t in (q._ema_cluster_size, q._ema_w):
+                dist.broadcast(t, src=src, group=self.group)
 
     # ---- gradient reduction: flat buffer, buckets reduced WHILE the backward pass is still running
     BUCKET_ELEMS = 8 * 1024 * 1024        # ~32 MB of fp32 per all-reduce: the decoder's last layer alone, then groups of smaller layers
@@ -171,9 +191,11 @@ class DataParallelTrainer(Trainer):
                     for bn in getattr(self, "_bn_modules", [])]
         for bn, _, _ in bn_saved:
             bn.lcrec_sync = None                                # the full batch is local in this pass
+        # an EMA model takes no EMA step in this pass: the first batch gets exactly one, in the training forward
+        kw = {"use_ema": False} if self._ema_levels() else {}
         try:
             with torch.no_grad():
-                self.model(data.to(self.device))
+                self.model(data.to(self.device), **kw)
         finally:
             for q, ds in saved:
                 q.dist_sinkhorn = ds
@@ -187,14 +209,20 @@ class DataParallelTrainer(Trainer):
                 dist.broadcast(q.embedding.weight.data, src=src, group=self.group)
 
     def _join_forward_collectives(self):
-        """A rank whose row block of this batch is empty still has to take part in the collectives of the forward pass: per
-        Sinkhorn level the 2-element MAX all-reduce of the centring and the in-kernel arrival of the marginal all-reduce
-        (both accept 0 local rows).  Skipping them would leave the peers' collectives mismatched with this rank's next one."""
-        for q in self._sinkhorn_levels:
-            d = torch.empty((0, q.n_e), dtype=torch.float32, device=self.device)
-            dc = q.dist_sinkhorn.center(d)
-            _, _, flags = q.dist_sinkhorn(dc, q.sk_epsilon, q.sk_iters)
-            ops.check_later("sinkhorn", flags)
+        """A rank whose row block of this batch is empty still has to take part in the collectives of the forward pass, in
+        the forward's level order: per Sinkhorn level the 2-element MAX all-reduce of the centring and the in-kernel arrival
+        of the marginal all-reduce, per EMA level the EMA step with 0 local rows (and the reset broadcast when it is due).
+        Skipping them would leave the peers' collectives mismatched with this rank's next one."""
+        rq = getattr(self.model, "rq", None)
+        for q in (rq.vq_layers if rq is not None else []):
+            if q in self._sinkhorn_levels:
+                d = torch.empty((0, q.n_e), dtype=torch.float32, device=self.device)
+                dc = q.dist_sinkhorn.center(d)
+                _, _, flags = q.dist_sinkhorn(dc, q.sk_epsilon, q.sk_iters)
+                ops.check_later("sinkhorn", flags)
+            if getattr(q, "dist_ema", None) is not None:
+                q.ema_step(torch.empty((0, q.e_dim), dtype=torch.float32, device=self.device),
+                           torch.empty((0,), dtype=torch.int64, device=self.device))
 
     def _train_epoch(self, train_data, epoch_idx):
         self.model.train()
@@ -209,6 +237,8 @@ class DataParallelTrainer(Trainer):
             weight = local.shape[0] / max(n, 1)
             for q in self._sinkhorn_levels:
                 q.dist_sinkhorn.n_rows_hint = n                 # the global row count, known here: no all-reduce + host read
+            if self._ema is not None:
+                self._ema.n_rows_hint = n
             if self._bn_modules:
                 if n < self.world:
                     raise RuntimeError(f"synchronised BatchNorm: a batch of {n} rows leaves a rank of {self.world} without rows")

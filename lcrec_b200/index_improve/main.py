@@ -1,6 +1,7 @@
 """Training CLI of the EMA variant: the flags of reference ``index_improve/main.py`` (:15-125) - those of ``index/main.py``
 plus --ema_decay / --epsilon / --reset_threshold / --reset_interval; ``--sk_epsilons`` defaults to zeros of the right
-length (:87-89).  The reference's default device ``npu:0`` becomes ``cuda:0`` (this library is sm_100a only)."""
+length (:87-89).  The reference's default device ``npu:0`` becomes ``cuda:0`` (this library is sm_100a only).  Under
+torchrun (WORLD_SIZE > 1) it trains data-parallel, one process per GPU, like ``lcrec_b200.main``."""
 import logging
 import random
 
@@ -9,9 +10,9 @@ import torch
 from torch.utils.data import DataLoader
 
 from ..datasets import EmbDataset
-from ..main import build_parser
+from ..main import build_parser, make_trainer
 from .models.rqvae import RQVAE
-from .trainer import Trainer
+from .trainer import DataParallelTrainer, Trainer
 
 
 def parse_args(argv=None):
@@ -49,7 +50,7 @@ def main(argv=None):
                   reset_interval=args.reset_interval)
     print(model)
     loader = DataLoader(data, num_workers=args.num_workers, batch_size=args.batch_size, shuffle=True, pin_memory=True)
-    best_loss, best_collision_rate = Trainer(args, model, len(loader)).fit(loader)
+    best_loss, best_collision_rate = make_trainer(args, model, len(loader), Trainer, DataParallelTrainer).fit(loader)
     print("=================================================")
     print("Training Completed!")
     print(f"Best Loss: {best_loss}")

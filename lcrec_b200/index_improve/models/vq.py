@@ -27,6 +27,9 @@ class VectorQuantizer(_BaseVectorQuantizer):
         self.step_count = 0
         self.register_buffer("_ema_cluster_size", torch.zeros(n_e))
         self.register_buffer("_ema_w", torch.zeros(n_e, e_dim))
+        # data-parallel training: a lcrec_b200.distributed.DistributedEma makes the EMA step ONE step over the global batch
+        # (the ranks' row blocks gathered through peer memory, identical buffers on every rank); None = local
+        self.dist_ema = None
 
     @torch.no_grad()
     def _reset_unused_codes(self, latent):
@@ -62,12 +65,41 @@ class VectorQuantizer(_BaseVectorQuantizer):
         if self.training and use_ema:
             # the gather above saved the indices, not the weights, so the in-place update cannot disturb backward
             # (the reference writes embedding.weight.data for the same reason)
-            ops.ema_update(latent.detach(), indices, self._ema_cluster_size, self._ema_w, self.embedding.weight.data,
+            self.ema_step(latent.detach(), indices)
+        return x_q, loss, indices.view(x.shape[:-1])
+
+    @torch.no_grad()
+    def ema_step(self, latent, indices):
+        """The EMA step, the step count and the dead-code reset when it is due (vq.py:146-187, :188-190).  Under
+        ``dist_ema`` the step runs over the global batch, and a rank whose block is empty still calls this with 0 rows."""
+        if self.dist_ema is None:
+            ops.ema_update(latent, indices, self._ema_cluster_size, self._ema_w, self.embedding.weight.data,
                            self.ema_decay, self.epsilon)
             self.step_count += 1
             if self.step_count % self.reset_interval == 0:
-                self._reset_unused_codes(latent.detach())
-        return x_q, loss, indices.view(x.shape[:-1])
+                self._reset_unused_codes(latent)
+            return
+        latent_global = self.dist_ema.update(latent, indices, None, self._ema_cluster_size, self._ema_w,
+                                             self.embedding.weight.data, self.ema_decay, self.epsilon)
+        self.step_count += 1
+        if self.step_count % self.reset_interval == 0:
+            self._reset_unused_codes_dist(latent_global)
+
+    @torch.no_grad()
+    def _reset_unused_codes_dist(self, latent_global):
+        """The reset over the global batch.  The dead codes follow from _ema_cluster_size, identical on every rank, so every
+        rank knows whether one happens; rank 0 then draws it (the reference's randint / randperm / randn_like sequence)
+        and broadcasts the level's buffers.  Replica equality never rests on the ranks' RNG states agreeing."""
+        import torch.distributed as dist
+        _, unused_mask = ops.codebook_usage(self._ema_cluster_size, self.epsilon, self.reset_threshold, want_unused=True)
+        if int(unused_mask.sum().item()) == 0 or len(latent_global) == 0:
+            return
+        group = self.dist_ema.group
+        if self.dist_ema.rank == 0:
+            self._reset_unused_codes(latent_global)
+        src = dist.get_global_rank(group, 0) if group is not dist.group.WORLD else 0
+        for t in (self.embedding.weight.data, self._ema_cluster_size, self._ema_w):
+            dist.broadcast(t, src=src, group=group)
 
     @torch.no_grad()
     def get_codebook_usage(self):

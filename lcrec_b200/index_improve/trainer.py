@@ -5,6 +5,7 @@ from __future__ import annotations
 
 import numpy as np
 
+from ..dp_trainer import DataParallelTrainer as _DataParallelTrainer
 from ..trainer import Trainer as _BaseTrainer
 from ..utils import set_color
 
@@ -30,3 +31,9 @@ class Trainer(_BaseTrainer):
                 out += (f"\n  Quantizer {stat['quantizer_id']}: {stat['utilization']:.4f} "
                         f"({stat['used_codes']}/{stat['total_codes']})")
         return out + "]"
+
+
+class DataParallelTrainer(_DataParallelTrainer, Trainer):
+    """Data-parallel training of the EMA variant over the GPUs of one box: the step of ``lcrec_b200.dp_trainer`` (one EMA
+    step per level over the global batch, see ``DistributedEma``) with this variant's ``use_ema=True`` forward and its
+    codebook-utilisation log."""

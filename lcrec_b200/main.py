@@ -41,6 +41,20 @@ def parse_args(argv=None):
     return build_parser().parse_args(argv)
 
 
+def make_trainer(args, model, data_num, trainer_cls, dp_trainer_cls):
+    """``trainer_cls`` on one device, or under torchrun (WORLD_SIZE > 1) ``dp_trainer_cls``: one process per GPU, every rank
+    reads the same batches and trains its row block of each."""
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    if world <= 1:
+        return trainer_cls(args, model, data_num)
+    import torch.distributed as dist
+    local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    torch.cuda.set_device(local_rank)
+    args.device = f"cuda:{local_rank}"
+    dist.init_process_group("nccl")
+    return dp_trainer_cls(args, model, data_num)
+
+
 def main(argv=None):
     seed = 2024
     random.seed(seed); np.random.seed(seed); torch.manual_seed(seed); torch.cuda.manual_seed_all(seed)
@@ -56,18 +70,8 @@ def main(argv=None):
                   kmeans_iters=args.kmeans_iters, sk_epsilons=args.sk_epsilons, sk_iters=args.sk_iters)
     print(model)
     loader = DataLoader(data, num_workers=args.num_workers, batch_size=args.batch_size, shuffle=True, pin_memory=True)
-    world = int(os.environ.get("WORLD_SIZE", "1"))
-    if world > 1:      # torchrun: one process per GPU, every rank reads the same batches and trains its row block of each
-        import torch.distributed as dist
-        from .dp_trainer import DataParallelTrainer
-        local_rank = int(os.environ.get("LOCAL_RANK", "0"))
-        torch.cuda.set_device(local_rank)
-        args.device = f"cuda:{local_rank}"
-        dist.init_process_group("nccl")
-        trainer = DataParallelTrainer(args, model, len(loader))
-    else:
-        trainer = Trainer(args, model, len(loader))
-    best_loss, best_collision_rate = trainer.fit(loader)
+    from .dp_trainer import DataParallelTrainer
+    best_loss, best_collision_rate = make_trainer(args, model, len(loader), Trainer, DataParallelTrainer).fit(loader)
     print("Best Loss", best_loss)
     print("Best Collision Rate", best_collision_rate)
 

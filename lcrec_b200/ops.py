@@ -105,14 +105,7 @@ _PENDING: List[Tuple[str, torch.Tensor]] = []
 
 
 def _evaluate_check(kind: str, word: torch.Tensor) -> None:
-    v = int(word.item())
-    if kind == "amplitude" and v != 0:
-        raise AssertionError("amplitude > 0")
-    if kind == "sinkhorn":
-        if v & 8:
-            raise RuntimeError("distributed Sinkhorn: a peer rank did not arrive")
-        if v & 1:
-            print("Sinkhorn Algorithm returns nan/inf values.")
+    evaluate_check_value(kind, int(word.item()))
 
 
 def check_later(kind: str, word: torch.Tensor) -> None:
@@ -138,6 +131,11 @@ def evaluate_check_value(kind: str, v: int) -> None:
             raise RuntimeError("distributed Sinkhorn: a peer rank did not arrive")
         if v & 1:
             print("Sinkhorn Algorithm returns nan/inf values.")
+    if kind == "ema_dist":
+        if v & 1:
+            raise RuntimeError("distributed EMA step: a peer rank did not arrive")
+        if v & 2:
+            raise RuntimeError("distributed EMA step: a peer published a row count other than its ShardPlan share")
 
 
 def flush_checks() -> None:
