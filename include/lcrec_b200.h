@@ -353,6 +353,17 @@ int lcrec_indexer_run_host_ex(lcrec_indexer_t* ix, const void* x_host, int dtype
 /* building blocks of the loop, for multi-GPU drivers and tests */
 int lcrec_indexer_pass0(lcrec_indexer_t* ix, const float* x, int64_t n, int64_t row_offset, void* stream);
 int lcrec_indexer_pass0_ex(lcrec_indexer_t* ix, const void* x, int dtype, int64_t n, int64_t row_offset, void* stream);
+/* PASS 0 of global rows [row_begin, row_begin + n) of an n_total-row job, read from host memory (pinned or pageable; x_host
+ * points at row row_begin) into table rows [0, n), streamed with the double-buffered copy of run_host.  The rows are cut along
+ * the pieces in which run_host streams n_total rows (a function of n_total and chunk_rows) and each part takes the RQ kernel
+ * path of its whole piece, so codes and last-level residuals are bit-identical to rows [row_begin, row_begin + n) of
+ * run_host's PASS 0 over all n_total rows: every rank of a sharded job computes exactly its rows of the one-GPU table.
+ * Returns once the host rows have been copied; the compute is ordered on `stream`, and the next call on the same indexer
+ * waits for it before reusing the staging buffers (no synchronisation needed between calls).  LCREC_ERR_ARG before any device work
+ * for row_begin < 0, row_begin + n > n_total, n > max_items or a dtype outside {0, 1, 2}.  run_host_ex is this entry with
+ * (n_total = n, row_begin = 0), then the rounds, then the copy of the codes. */
+int lcrec_indexer_pass0_host_ex(lcrec_indexer_t* ix, const void* x_host, int dtype, int64_t n_total, int64_t row_begin,
+                                int64_t n, void* stream);
 int lcrec_indexer_round(lcrec_indexer_t* ix, int64_t n, int64_t* counts_host, void* stream);
 /* The collision rounds alone (generate_indices.py:108-128) on caller-owned device arrays: codes (n, L) int64 updated
  * in place, resid (n, e_dim) = residual entering the last level; n <= max_items.  stats_host as in run_host. */
@@ -445,6 +456,12 @@ int lcrec_masked_mean_pool(const void* hidden, int dtype, const int64_t* mask, i
 int64_t lcrec_index_json_workspace_bytes(int64_t n);
 int lcrec_index_json(const int64_t* codes, int64_t n, int n_levels, char* out, int64_t out_cap, int64_t* total_bytes_dev,
                      void* ws, int64_t ws_bytes, void* stream);
+/* The same text for a block of rows: row i has the key item_base + i (int64), ", " goes in front of every row whose key is
+ * not 0, and braces (0 / 1) selects whether "{" and "}" are written.  "{" + the fragments (braces 0) of consecutive blocks +
+ * "}" is the text of the whole table, so each rank of a sharded job formats its rows on its own device and writes them at
+ * their offset.  lcrec_index_json is (item_base 0, braces 1). */
+int lcrec_index_json_ex(const int64_t* codes, int64_t n, int n_levels, int64_t item_base, int braces, char* out,
+                        int64_t out_cap, int64_t* total_bytes_dev, void* ws, int64_t ws_bytes, void* stream);
 /* ---- (e) multi-GPU hand-over of PASS-0 results to the owners of the prefix buckets (lcrec_b200/distributed.py) -----------
  * pack: owner = hash(first L-1 codes) mod world; STABLE partition of this rank's n items by owner straight into `send` =
  * `world` slabs of lcrec_exchange_slab_bytes(slab_rows, L, D) bytes: [16 B header: int64 row count, int64 overflow flag][records:

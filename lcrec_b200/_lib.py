@@ -80,6 +80,7 @@ SIGNATURES = {
     "lcrec_indexer_run_device_ex": (C.c_int, [vp, vp, C.c_int, i64, C.c_int, vp, C.POINTER(i64), vp]),
     "lcrec_indexer_run_host_ex": (C.c_int, [vp, vp, C.c_int, i64, C.c_int, vp, C.POINTER(i64), vp]),
     "lcrec_indexer_pass0_ex": (C.c_int, [vp, vp, C.c_int, i64, i64, vp]),
+    "lcrec_indexer_pass0_host_ex": (C.c_int, [vp, vp, C.c_int, i64, i64, i64, vp]),
     "lcrec_indexer_round": (C.c_int, [vp, i64, C.POINTER(i64), vp]),
     "lcrec_indexer_resolve": (C.c_int, [vp, vp, vp, i64, C.c_int, C.POINTER(i64), vp]),
     "lcrec_indexer_set_segments": (C.c_int, [C.c_int]),
@@ -115,6 +116,7 @@ SIGNATURES = {
     "lcrec_recon_loss_backward": (C.c_int, [vp, vp, i64, C.c_int, vp, vp, vp]),
     "lcrec_index_json_workspace_bytes": (i64, [i64]),
     "lcrec_index_json": (C.c_int, [vp, i64, C.c_int, vp, i64, vp, vp, i64, vp]),
+    "lcrec_index_json_ex": (C.c_int, [vp, i64, C.c_int, i64, C.c_int, vp, i64, vp, vp, i64, vp]),
     "lcrec_fp64_peak_probe": (C.c_int, [C.POINTER(f64), vp, i64, vp]),
     "lcrec_ddiv_probe": (C.c_int, [vp, vp, i64, vp, vp]),
     "lcrec_sinkhorn_set_col": (C.c_int, [C.c_int]),

@@ -243,24 +243,93 @@ extern "C" int lcrec_indexer_destroy(lcrec_indexer_t* ix) {
 extern "C" int64_t* lcrec_indexer_codes(lcrec_indexer_t* ix) { return ix ? ix->codes : nullptr; }
 extern "C" float* lcrec_indexer_resid(lcrec_indexer_t* ix) { return ix ? ix->resid : nullptr; }
 
-// PASS 0 for rows [row_offset, row_offset + n) (generate_indices.py:85-95); x of element type dtype
-extern "C" int lcrec_indexer_pass0_ex(lcrec_indexer_t* ix, const void* x, int dtype, int64_t n, int64_t row_offset, void* stream) {
-  LC_ARG(dtype_ok(dtype));
-  LC_ARG(ix && n >= 0 && row_offset >= 0 && row_offset + n <= ix->max_items);
-  if (n == 0) return LCREC_OK;
-  LC_ARG(x != nullptr);
+namespace lcrec {
+int rq_quantize_select(const float* z, int64_t n, int64_t n_select, int e_dim, int n_levels, const float* const* codebooks,
+                       const int32_t* n_codes, int n_levels_run, int resid_level, int64_t* codes, float* xq, float* resid_last,
+                       double* sq_err, void* stream);      // rq_fused.cu
+}
+
+// PASS 0 of n device rows into table rows [row_offset, row_offset + n), the RQ kernel path chosen as for n_select rows
+static int pass0_rows(lcrec_indexer_t* ix, const void* x, int dtype, int64_t n, int64_t row_offset, int64_t n_select,
+                      void* stream) {
   const int64_t row_bytes = dtype_bytes(dtype) * ix->in_dim;
   for (int64_t s = 0; s < n; s += ix->chunk_rows) {
     const int64_t m = std::min(ix->chunk_rows, n - s);
     LC_TRY(lcrec_mlp_forward_ex(ix->enc, static_cast<const char*>(x) + s * row_bytes, dtype, m, ix->z + s * ix->D, nullptr,
                                 ix->mlp_ws, ix->mlp_ws_bytes, stream));
   }
-  {
-    ProfScope prof(20, (cudaStream_t)stream);
-    LC_TRY(lcrec_rq_quantize(ix->z, n, ix->D, ix->L, ix->cb.data(), ix->K.data(), ix->L, ix->L - 1,
-                             ix->codes + row_offset * ix->L, nullptr, ix->resid + row_offset * ix->D,
-                             nullptr, stream));
+  ProfScope prof(20, (cudaStream_t)stream);
+  return rq_quantize_select(ix->z, n, n_select, ix->D, ix->L, ix->cb.data(), ix->K.data(), ix->L, ix->L - 1,
+                            ix->codes + row_offset * ix->L, nullptr, ix->resid + row_offset * ix->D, nullptr, stream);
+}
+
+// PASS 0 for rows [row_offset, row_offset + n) (generate_indices.py:85-95); x of element type dtype
+extern "C" int lcrec_indexer_pass0_ex(lcrec_indexer_t* ix, const void* x, int dtype, int64_t n, int64_t row_offset, void* stream) {
+  LC_ARG(dtype_ok(dtype));
+  LC_ARG(ix && n >= 0 && row_offset >= 0 && row_offset + n <= ix->max_items);
+  if (n == 0) return LCREC_OK;
+  LC_ARG(x != nullptr);
+  return pass0_rows(ix, x, dtype, n, row_offset, n, stream);
+}
+
+// The pieces in which host input of n_total rows is streamed: chunks of chunk_rows rows, the last chunk cut into up to four
+// pieces (>= 8192 rows each).  The copies are the bottleneck (55 GB/s of pinned H2D against ~14 M items/s of compute), so
+// what is left after the LAST copy lands - that chunk's encoder pass - is pure tail: cutting it leaves only a quarter of it
+// to encode when the link goes idle.  Every piece keeps >= 8192 rows, so it gets the same kernel choices as a full chunk
+// (tensor-core RQ path from 4096 rows on).  A pure function of (n_total, chunk_rows): a block of a larger job is cut along
+// the same pieces (lcrec_indexer_pass0_host_ex).
+static void host_pieces(int64_t n_total, int64_t chunk_rows, std::vector<std::pair<int64_t, int64_t>>& pieces) {
+  pieces.clear();
+  for (int64_t s0 = 0; s0 < n_total; s0 += chunk_rows) {
+    const int64_t m0 = std::min(chunk_rows, n_total - s0);
+    if (s0 + m0 < n_total) { pieces.emplace_back(s0, m0); continue; }
+    const int64_t k = std::max<int64_t>(1, std::min<int64_t>(4, m0 / 8192));
+    const int64_t q = ceil_div(m0, k);
+    for (int64_t t = 0; t < m0; t += q) pieces.emplace_back(s0 + t, std::min(q, m0 - t));
   }
+}
+
+// PASS 0 of global rows [row_begin, row_begin + n) of an n_total-row job from host memory into table rows [0, n):
+// double-buffered H2D on the indexer's copy stream, compute on `stream` (the fp32-sized staging buffers also hold a piece of
+// half rows).  The block is cut along the pieces of host_pieces(n_total, chunk_rows) and every part is quantised with the
+// RQ path of its whole piece, so codes and residuals are bit-identical to those rows of the single-call PASS 0 over all
+// n_total rows.  Returns once every row has been copied; the compute stays ordered on `stream`.
+extern "C" int lcrec_indexer_pass0_host_ex(lcrec_indexer_t* ix, const void* x_host, int dtype, int64_t n_total, int64_t row_begin,
+                                           int64_t n, void* stream) {
+  LC_ARG(dtype_ok(dtype));
+  LC_ARG(ix && n >= 0 && row_begin >= 0 && n_total >= 0 && row_begin <= n_total && n <= n_total - row_begin && n <= ix->max_items);
+  if (n == 0) return LCREC_OK;
+  LC_ARG(x_host != nullptr);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (!ix->copy_stream) {
+    LC_CUDA(cudaStreamCreateWithFlags(&ix->copy_stream, cudaStreamNonBlocking));
+    for (int i = 0; i < 2; ++i) {
+      LC_CUDA(cudaEventCreateWithFlags(&ix->ev_copied[i], cudaEventDisableTiming));
+      LC_CUDA(cudaEventCreateWithFlags(&ix->ev_consumed[i], cudaEventDisableTiming));
+      LC_CUDA(cudaMalloc((void**)&ix->stage[i], sizeof(float) * ix->chunk_rows * ix->in_dim));
+    }
+  }
+  std::vector<std::pair<int64_t, int64_t>> pieces;
+  host_pieces(n_total, ix->chunk_rows, pieces);
+  const int64_t row_bytes = dtype_bytes(dtype) * ix->in_dim;
+  const int64_t end = row_begin + n;
+  int64_t c = 0;      // parts streamed so far
+  for (const auto& pc : pieces) {
+    const int64_t s = std::max(pc.first, row_begin), e = std::min(pc.first + pc.second, end);
+    if (s >= e) continue;
+    const int b = (int)(c & 1);
+    // also for the first two parts: the previous call's last passes over stage[b] may still be queued on `stream` (this
+    // entry returns once the copies land, not the compute); an event never recorded counts as complete
+    LC_CUDA(cudaStreamWaitEvent(ix->copy_stream, ix->ev_consumed[b], 0));
+    LC_CUDA(cudaMemcpyAsync(ix->stage[b], static_cast<const char*>(x_host) + (s - row_begin) * row_bytes, (e - s) * row_bytes,
+                            cudaMemcpyHostToDevice, ix->copy_stream));
+    LC_CUDA(cudaEventRecord(ix->ev_copied[b], ix->copy_stream));
+    LC_CUDA(cudaStreamWaitEvent(st, ix->ev_copied[b], 0));
+    LC_TRY(pass0_rows(ix, ix->stage[b], dtype, e - s, s - row_begin, pc.second, stream));
+    LC_CUDA(cudaEventRecord(ix->ev_consumed[b], st));
+    ++c;
+  }
+  LC_CUDA(cudaStreamSynchronize(ix->copy_stream));      // the caller's host rows may be released on return
   return LCREC_OK;
 }
 
@@ -525,38 +594,7 @@ extern "C" int lcrec_indexer_run_host_ex(lcrec_indexer_t* ix, const void* x_host
   cudaStream_t st = (cudaStream_t)stream;
   if (n == 0) { if (stats_host) memset(stats_host, 0, 8 * sizeof(int64_t)); return LCREC_OK; }
   LC_ARG(x_host && codes_host);
-  if (!ix->copy_stream) {
-    LC_CUDA(cudaStreamCreateWithFlags(&ix->copy_stream, cudaStreamNonBlocking));
-    for (int i = 0; i < 2; ++i) {
-      LC_CUDA(cudaEventCreateWithFlags(&ix->ev_copied[i], cudaEventDisableTiming));
-      LC_CUDA(cudaEventCreateWithFlags(&ix->ev_consumed[i], cudaEventDisableTiming));
-      LC_CUDA(cudaMalloc((void**)&ix->stage[i], sizeof(float) * ix->chunk_rows * ix->in_dim));
-    }
-  }
-  // double-buffered H2D on the copy stream, compute on `st` (the fp32-sized staging buffers also hold a piece of half rows).  The copies are the bottleneck (55 GB/s of pinned H2D against ~14 M
-  // items/s of compute), so what is left after the LAST copy lands - that chunk's encoder pass - is pure tail: the last chunk is cut
-  // into up to four pieces (>= 8192 rows each) so that only a quarter of it remains to be encoded when the link goes idle.
-  std::vector<std::pair<int64_t, int64_t>> pieces;
-  for (int64_t s0 = 0; s0 < n; s0 += ix->chunk_rows) {
-    const int64_t m0 = std::min(ix->chunk_rows, n - s0);
-    if (s0 + m0 < n) { pieces.emplace_back(s0, m0); continue; }
-    const int64_t k = std::max<int64_t>(1, std::min<int64_t>(4, m0 / 8192));      // every piece keeps >= 8192 rows: same kernel choices
-    const int64_t q = ceil_div(m0, k);                                            // (tensor-core RQ path from 4096 rows on) as a full chunk
-    for (int64_t t = 0; t < m0; t += q) pieces.emplace_back(s0 + t, std::min(q, m0 - t));
-  }
-  const int64_t nchunks = (int64_t)pieces.size();
-  const int64_t row_bytes = dtype_bytes(dtype) * ix->in_dim;
-  for (int64_t c = 0; c < nchunks; ++c) {
-    const int b = (int)(c & 1);
-    const int64_t s = pieces[c].first, m = pieces[c].second;
-    if (c >= 2) LC_CUDA(cudaStreamWaitEvent(ix->copy_stream, ix->ev_consumed[b], 0));
-    LC_CUDA(cudaMemcpyAsync(ix->stage[b], static_cast<const char*>(x_host) + s * row_bytes, m * row_bytes,
-                            cudaMemcpyHostToDevice, ix->copy_stream));
-    LC_CUDA(cudaEventRecord(ix->ev_copied[b], ix->copy_stream));
-    LC_CUDA(cudaStreamWaitEvent(st, ix->ev_copied[b], 0));
-    LC_TRY(lcrec_indexer_pass0_ex(ix, ix->stage[b], dtype, m, s, stream));
-    LC_CUDA(cudaEventRecord(ix->ev_consumed[b], st));
-  }
+  LC_TRY(lcrec_indexer_pass0_host_ex(ix, x_host, dtype, n, 0, n, stream));
   LC_TRY(indexer_rounds(ix, n, max_rounds, stats_host, st));
   LC_CUDA(cudaMemcpyAsync(codes_host, ix->codes, sizeof(int64_t) * n * ix->L, cudaMemcpyDeviceToHost, st));
   LC_CUDA(cudaStreamSynchronize(st));

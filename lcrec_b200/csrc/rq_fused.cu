@@ -505,11 +505,11 @@ static int launch_rq_smem_impl(const RqArgs& a, size_t smem, cudaStream_t st) {
   return LCREC_OK;
 }
 template <int D>
-static int launch_rq_smem(const RqArgs& a, size_t smem, cudaStream_t st) {
+static int launch_rq_smem(const RqArgs& a, int64_t n_select, size_t smem, cudaStream_t st) {
   if (a.xq != nullptr || a.sq_err != nullptr) return launch_rq_smem_impl<D, 1, true, 256>(a, smem, st);
   if constexpr (D <= 32) {
-    if (a.n >= 4096) {
-      if (g_rq_ipt == 4 && a.n >= 65536) return launch_rq_smem_impl<D, 4, false, 256>(a, smem, st);
+    if (n_select >= 4096) {
+      if (g_rq_ipt == 4 && n_select >= 65536) return launch_rq_smem_impl<D, 4, false, 256>(a, smem, st);
       return launch_rq_smem_impl<D, 2, false, 512>(a, smem, st);
     }
   }
@@ -530,10 +530,14 @@ extern "C" int lcrec_rq_set_tc_mode(int mode) {
   return LCREC_OK;
 }
 
-extern "C" int lcrec_rq_quantize(const float* z, int64_t n, int e_dim, int n_levels, const float* const* codebooks,
-                                 const int32_t* n_codes, int n_levels_run, int resid_level, int64_t* codes,
-                                 float* xq, float* resid_last, double* sq_err, void* stream) {
-  LC_ARG(n >= 0 && e_dim > 0 && n_levels >= 1 && n_levels <= LCREC_MAX_LEVELS && codebooks && n_codes);
+namespace lcrec {
+// lcrec_rq_quantize with the kernel path chosen as if the call had n_select rows (n_select >= n).  The tensor-core and SIMT
+// paths agree only up to near-ties, so a caller that quantises part of a larger batch passes the batch's row count to get
+// the codes the whole batch would get (lcrec_indexer_pass0_host_ex).  lcrec_rq_quantize is n_select = n.
+int rq_quantize_select(const float* z, int64_t n, int64_t n_select, int e_dim, int n_levels, const float* const* codebooks,
+                       const int32_t* n_codes, int n_levels_run, int resid_level, int64_t* codes, float* xq, float* resid_last,
+                       double* sq_err, void* stream) {
+  LC_ARG(n >= 0 && n_select >= n && e_dim > 0 && n_levels >= 1 && n_levels <= LCREC_MAX_LEVELS && codebooks && n_codes);
   LC_ARG(n_levels_run >= 0 && n_levels_run <= n_levels);
   LC_TRY(lcrec_device_check());
   if (n == 0) return LCREC_OK;
@@ -553,16 +557,16 @@ extern "C" int lcrec_rq_quantize(const float* z, int64_t n, int e_dim, int n_lev
   bool cb_aligned = true;
   for (int l = 0; l < n_levels_run; ++l) cb_aligned = cb_aligned && (reinterpret_cast<uintptr_t>(codebooks[l]) & 15) == 0;
   // tensor-core distance path (CTA-pair GEMM + argmin epilogue) for the shapes it serves
-  bool tc_ok = codes != nullptr && n_levels_run > 0 && g_rq_tc_mode != 0 && n >= 1024, tc_big = false;
+  bool tc_ok = codes != nullptr && n_levels_run > 0 && g_rq_tc_mode != 0 && n_select >= 1024, tc_big = false;
   for (int l = 0; l < n_levels_run; ++l) { tc_ok = tc_ok && argmin_pair_supported(e_dim, n_codes[l]); tc_big = tc_big || n_codes[l] >= 4096; }
   if (tc_ok && g_rq_tc_mode == 2) return rq_quantize_tc(a, e_dim, st);
   // small e_dim with 256-multiple codebooks: the tensor-core path (thread-per-row prepare + CTA-pair distance GEMM) is
   // 1.7x the SIMT kernel from a few thousand rows on (1 M items, 4 x 256 x 32: 1.43 vs 2.38 ms)
-  if (tc_ok && n >= 4096 && (e_dim == 16 || e_dim == 32 || e_dim == 64) && aligned && cb_aligned) return rq_quantize_tc(a, e_dim, st);
+  if (tc_ok && n_select >= 4096 && (e_dim == 16 || e_dim == 32 || e_dim == 64) && aligned && cb_aligned) return rq_quantize_tc(a, e_dim, st);
   if (smem <= 200 * 1024 && aligned && cb_aligned && n_levels_run > 0) {
-    if (e_dim == 32) return launch_rq_smem<32>(a, smem, st);
-    if (e_dim == 16) return launch_rq_smem<16>(a, smem, st);
-    if (e_dim == 64) return launch_rq_smem<64>(a, smem, st);
+    if (e_dim == 32) return launch_rq_smem<32>(a, n_select, smem, st);
+    if (e_dim == 16) return launch_rq_smem<16>(a, n_select, smem, st);
+    if (e_dim == 64) return launch_rq_smem<64>(a, n_select, smem, st);
   }
   if (tc_ok && (tc_big || e_dim >= 128)) return rq_quantize_tc(a, e_dim, st);
   // generic path
@@ -580,6 +584,14 @@ extern "C" int lcrec_rq_quantize(const float* z, int64_t n, int e_dim, int n_lev
   LC_LAUNCH_CHECK("rq_quantize_generic_kernel");
   LC_CUDA(cudaFreeAsync(norms, st));
   return LCREC_OK;
+}
+}  // namespace lcrec
+
+extern "C" int lcrec_rq_quantize(const float* z, int64_t n, int e_dim, int n_levels, const float* const* codebooks,
+                                 const int32_t* n_codes, int n_levels_run, int resid_level, int64_t* codes,
+                                 float* xq, float* resid_last, double* sq_err, void* stream) {
+  return rq_quantize_select(z, n, n, e_dim, n_levels, codebooks, n_codes, n_levels_run, resid_level, codes, xq, resid_last,
+                            sq_err, stream);
 }
 
 extern "C" int lcrec_vq_distances(const float* r, int64_t n, int e_dim, const float* codebook, int n_codes,

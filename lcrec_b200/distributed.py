@@ -66,26 +66,35 @@ def all_gather_rows(local: torch.Tensor, plan: ShardPlan, rank: int, group=None)
 class CudaBackend:
     """Kernels of liblcrec_b200.so on this rank's GPU."""
 
-    def __init__(self, model, n_local_max: int, chunk_rows: int = 131072):
+    def __init__(self, model, n_local_max: int, chunk_rows: int = 131072, n_total: int = None):
+        """``n_total``: the rows of the whole job, for ranks that read host blocks (``pass0`` with a layout): the indexer then
+        streams in the pieces of the one-GPU run over n_total rows (chunks of min(chunk_rows, n_total) rows)."""
         from . import generate_indices as G
         from . import ops
         self.ops = ops
         self.model = model
+        chunk = min(chunk_rows, max(n_local_max if n_total is None else n_total, 1))
         # 5 % slack: the hash-balanced bucket share of a rank may slightly exceed its item share
-        self.indexer = G.build_indexer(model, int(max(n_local_max, 1) * 1.05) + 1024, min(chunk_rows, max(n_local_max, 1)))
+        self.indexer = G.build_indexer(model, max(int(max(n_local_max, 1) * 1.05) + 1024, chunk), chunk)
         self.cbs = [vq.embedding.weight.detach() for vq in model.rq.vq_layers]
         self.n_codes = [int(c.shape[0]) for c in self.cbs]
         self.eps = float(model.rq.vq_layers[-1].sk_epsilon)
         self.iters = int(model.rq.vq_layers[-1].sk_iters)
 
-    def pass0(self, x_local: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
-        """Codes + last-level residuals of this rank's shard; an fp16 / bf16 shard is read as it is (Indexer.pass0)."""
+    def pass0(self, x_local, n_total: int = None, row_begin: int = 0) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Codes + last-level residuals of this rank's shard; an fp16 / bf16 shard is read as it is.  A CUDA tensor goes
+        through Indexer.pass0; a host block (CPU tensor or ndarray, e.g. a slice of an ``np.memmap``) is streamed from the
+        host as rows [row_begin, row_begin + n) of an ``n_total``-row job (Indexer.pass0_host), so its codes are those of
+        the one-GPU run over all n_total rows, bit for bit."""
         n = x_local.shape[0]
         if n == 0:
             dev = self.cbs[0].device
             return (torch.zeros((0, len(self.cbs)), dtype=torch.int64, device=dev),
                     torch.zeros((0, self.cbs[0].shape[1]), dtype=torch.float32, device=dev))
-        self.indexer.pass0(x_local, 0)
+        if isinstance(x_local, torch.Tensor) and x_local.is_cuda:
+            self.indexer.pass0(x_local, 0)
+        else:
+            self.indexer.pass0_host(x_local, n if n_total is None else n_total, row_begin)
         return self.indexer.codes_view(n).clone(), self.indexer.resid_view(n).clone()
 
     def collisions(self, codes: torch.Tensor) -> dict:
@@ -128,6 +137,7 @@ class NativeExchange:
         self.back_send = torch.empty((world, self.slab_rows), dtype=torch.int64, device=dev)
         self.back_recv = torch.empty_like(self.back_send)
         self.slot = torch.empty(max(n_local_max, 1), dtype=torch.int32, device=dev)
+        self.counts = torch.empty(world, dtype=torch.int64, device=dev)
         self.ws = torch.empty(int(self.lib.lcrec_exchange_workspace_bytes(max(n_local_max, 1), world)), dtype=torch.uint8, device=dev)
         self.cap = world * self.slab_rows
         self.sub_codes = torch.empty((self.cap, self.L), dtype=torch.int64, device=dev)
@@ -137,19 +147,24 @@ class NativeExchange:
         return self.C.c_void_p(torch.cuda.current_stream(self.dev).cuda_stream)
 
     def forward(self, codes_local: torch.Tensor, resid_local: torch.Tensor):
-        """-> (sub_codes view, sub_resid view) of the rows this rank owns, in ascending global item order."""
+        """-> (sub_codes view, sub_resid view) of the rows this rank owns, in ascending global item order; None on EVERY
+        rank when a destination slab of ANY rank overflowed (bucket skew beyond the 25 % slack): whether one did is
+        all-reduced before the slabs move, so all ranks take the split-size path together and none waits in a collective
+        that a failed peer never joins.  Collective."""
         from . import _lib
         from .ops import _p
         n = int(codes_local.shape[0])
         assert n <= self.slot.numel()
         with torch.cuda.device(self.dev):
             _lib.check(self.lib.lcrec_exchange_pack(_p(codes_local), _p(resid_local), n, self.L, self.D, self.n_codes, self.world,
-                                                    self.slab_rows, _p(self.send), _p(self.slot), None, _p(self.ws), self.ws.numel(), self._st()))
+                                                    self.slab_rows, _p(self.send), _p(self.slot), _p(self.counts), _p(self.ws),
+                                                    self.ws.numel(), self._st()))
+            overflow = (self.counts > self.slab_rows).any().to(torch.int32).view(1)
+            dist.all_reduce(overflow, op=dist.ReduceOp.MAX, group=self.group)
+            if int(overflow.item()) != 0:
+                return None
             dist.all_to_all_single(self.recv, self.send, group=self.group)
-            hdr = self.recv.view(self.world, self.slab_bytes)[:, :16].contiguous().view(torch.int64).cpu()      # the one host read
-            if int(hdr[:, 1].sum()) != 0:
-                raise RuntimeError("prefix-bucket exchange: a destination slab overflowed (bucket skew beyond 25 %); "
-                                   "set LCREC_EXCHANGE=generic for the split-size path")
+            hdr = self.recv.view(self.world, self.slab_bytes)[:, :16].contiguous().view(torch.int64).cpu()
             n_mine = int(hdr[:, 0].sum())
             _lib.check(self.lib.lcrec_exchange_unpack(_p(self.recv), self.world, self.slab_rows, self.L, self.D, _p(self.sub_codes),
                                                       _p(self.sub_resid), n_mine, self._st()))
@@ -206,7 +221,8 @@ def generate_codes_sharded(backend, x_local: torch.Tensor, plan: ShardPlan, rank
     """Sharded ``generate_indices``: returns (codes of this rank's items, stats).  Collective: every
     rank of ``group`` must call it."""
     import os
-    timing = os.environ.get("LCREC_DIST_TIMING") == "1" and x_local.is_cuda
+    on_device = isinstance(x_local, torch.Tensor) and x_local.is_cuda
+    timing = os.environ.get("LCREC_DIST_TIMING") == "1" and (on_device or isinstance(backend, CudaBackend))
     marks = []
 
     def mark(name):
@@ -215,7 +231,11 @@ def generate_codes_sharded(backend, x_local: torch.Tensor, plan: ShardPlan, rank
             e.record()
             marks.append((name, e))
     mark("start")
-    codes_local, resid_local = backend.pass0(x_local)
+    if not on_device and isinstance(backend, CudaBackend):
+        # a host block: streamed in the pieces of the one-GPU run over all plan.n_total rows
+        codes_local, resid_local = backend.pass0(x_local, plan.n_total, plan.start(rank))
+    else:
+        codes_local, resid_local = backend.pass0(x_local)
     mark("pass0")
     n_codes = n_codes or getattr(backend, "n_codes")
     if plan.world == 1:
@@ -234,7 +254,11 @@ def generate_codes_sharded(backend, x_local: torch.Tensor, plan: ShardPlan, rank
         if ex is None or ex.world != world or ex.slot.numel() < codes_local.shape[0] or getattr(backend, "_native_exchange_group", None) is not group:
             ex = backend._native_exchange = NativeExchange(backend, max(plan.max_count, int(codes_local.shape[0])), world, group)
             backend._native_exchange_group = group
-        sub_codes, sub_resid = ex.forward(codes_local.contiguous(), resid_local.contiguous())
+        fwd = ex.forward(codes_local.contiguous(), resid_local.contiguous())
+    else:
+        fwd = None
+    if fwd is not None:
+        sub_codes, sub_resid = fwd
         mark("partition+exchange")
         st = resolve_rounds(backend, sub_codes, sub_resid, max_rounds)
         mark("rounds")
@@ -248,13 +272,11 @@ def generate_codes_sharded(backend, x_local: torch.Tensor, plan: ShardPlan, rank
         n_unique, g1, r1, rows = [int(v) for v in gl[:, :4].sum(0).tolist()]
         rounds, max_mult = [int(v) for v in gl[:, 4:].max(0).values.tolist()]
         mark("return+stats")
-        if timing and rank == 0:
-            torch.cuda.synchronize()
-            import sys
-            print("dist timing (ms): " + ", ".join(f"{b[0]} {a[1].elapsed_time(b[1]):.2f}" for a, b in zip(marks[:-1], marks[1:])), file=sys.stderr)
         stats = {"rounds": rounds, "n_unique": n_unique, "groups_round1": g1, "rows_round1": r1, "sinkhorn_rows": rows,
                  "max_multiplicity": max_mult, "collision_rate": (plan.n_total - n_unique) / max(plan.n_total, 1),
                  "bucket_items_this_rank": n_mine}
+        if timing:
+            stats["timing_ms"] = _report_marks(marks, rank)
         return out, stats
     owner = bucket_owner(codes_local, n_codes, world)
     order = torch.argsort(owner, stable=True)                      # items grouped by destination, ascending inside
@@ -284,14 +306,22 @@ def generate_codes_sharded(backend, x_local: torch.Tensor, plan: ShardPlan, rank
     n_unique, g1, r1, rows = [int(v) for v in agg.tolist()]
     rounds, max_mult = [int(v) for v in mx.tolist()]
     mark("return+stats")
-    if timing and rank == 0:
-        torch.cuda.synchronize()
-        import sys
-        print("dist timing (ms): " + ", ".join(f"{b[0]} {a[1].elapsed_time(b[1]):.2f}" for a, b in zip(marks[:-1], marks[1:])), file=sys.stderr)
     stats = {"rounds": rounds, "n_unique": n_unique, "groups_round1": g1, "rows_round1": r1, "sinkhorn_rows": rows,
              "max_multiplicity": max_mult, "collision_rate": (plan.n_total - n_unique) / max(plan.n_total, 1),
              "bucket_items_this_rank": n_mine}
+    if timing:
+        stats["timing_ms"] = _report_marks(marks, rank)
     return out, stats
+
+
+def _report_marks(marks, rank: int) -> dict:
+    """LCREC_DIST_TIMING=1: ms between consecutive marks of generate_codes_sharded (printed by rank 0 to stderr)."""
+    torch.cuda.synchronize()
+    ms = {b[0]: a[1].elapsed_time(b[1]) for a, b in zip(marks[:-1], marks[1:])}
+    if rank == 0:
+        import sys
+        print("dist timing (ms): " + ", ".join(f"{k} {v:.2f}" for k, v in ms.items()), file=sys.stderr)
+    return ms
 
 
 # ----------------------------------------------------------------------------------------------------------------

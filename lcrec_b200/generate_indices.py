@@ -15,6 +15,8 @@ from __future__ import annotations
 import argparse
 import json
 import os
+import sys
+import time
 from typing import Optional
 
 import numpy as np
@@ -88,11 +90,45 @@ def write_index_json(codes, output_file: str) -> None:
         json.dump(codes_to_index_dict(codes), fp)                  # generate_indices.py:144-145
 
 
-def load_model(ckpt_path: str, device, in_dim: Optional[int] = None, data_path: Optional[str] = None):
-    """generate_indices.py:51-74 (``weights_only=False``: the checkpoint pickles an argparse.Namespace)."""
+def write_index_json_parts(fragment: bytes, output_file: str, group=None) -> None:
+    """Collective: the `.index.json` of a table whose row blocks are spread over the ranks of ``group`` in rank order, from
+    each rank's fragment (``ops.index_json_bytes(codes, item_base, braces=False)``).  One all-gather of the fragment lengths
+    gives every rank its byte offset; rank 0 creates the file at its final size and writes the braces, then every rank
+    writes its bytes in place with one positional write (the ranks share one host's file system)."""
+    import torch.distributed as dist
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    dev = torch.device("cuda", torch.cuda.current_device()) if dist.get_backend(group) == "nccl" else torch.device("cpu")
+    lens = torch.empty(world, dtype=torch.int64, device=dev)
+    dist.all_gather_into_tensor(lens, torch.tensor([len(fragment)], dtype=torch.int64, device=dev), group=group)
+    lens = lens.tolist()
+    total = 2 + sum(lens)
+    if rank == 0:
+        fd = os.open(output_file, os.O_WRONLY | os.O_CREAT | os.O_TRUNC, 0o666)
+        try:
+            os.ftruncate(fd, total)
+            os.pwrite(fd, b"{", 0)
+            os.pwrite(fd, b"}", total - 1)
+        finally:
+            os.close(fd)
+    dist.barrier(group=group)                                  # the file exists at its size before anyone writes into it
+    if fragment:
+        fd = os.open(output_file, os.O_WRONLY)
+        try:
+            view, off = memoryview(fragment), 1 + sum(lens[:rank])
+            while view:                                         # pwrite may write less than asked
+                k = os.pwrite(fd, view, off)
+                view, off = view[k:], off + k
+        finally:
+            os.close(fd)
+    dist.barrier(group=group)                                  # the file is complete when any rank returns
+
+
+def load_model(ckpt_path: str, device, in_dim: Optional[int] = None, data_path: Optional[str] = None, mmap: bool = False):
+    """generate_indices.py:51-74 (``weights_only=False``: the checkpoint pickles an argparse.Namespace).  ``mmap``: the
+    embeddings are a read-only memory map of the ``.npy`` instead of a copy in host memory."""
     ckpt = torch.load(ckpt_path, map_location=torch.device("cpu"), weights_only=False)
     args = ckpt["args"]
-    data = EmbDataset(data_path or args.data_path)
+    data = EmbDataset(data_path or args.data_path, mmap=mmap)
     model = RQVAE(in_dim=in_dim or data.dim, num_emb_list=args.num_emb_list, e_dim=args.e_dim, layers=args.layers,
                   dropout_prob=args.dropout_prob, bn=args.bn, loss_type=args.loss_type,
                   quant_loss_weight=args.quant_loss_weight, kmeans_init=args.kmeans_init,
@@ -110,18 +146,88 @@ def main(argv=None):
     ap.add_argument("--device", default="cuda:0")
     ap.add_argument("--max_rounds", type=int, default=20)
     ap.add_argument("--chunk_rows", type=int, default=131072)
+    ap.add_argument("--dist_timeout", type=float, default=1800.0,
+                    help="seconds a rank waits in a collective before it fails (under torchrun)")
     a = ap.parse_args(argv)
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    if world > 1:
+        return _main_sharded(a, world)
     device = torch.device(a.device)
+    timing = os.environ.get("LCREC_DIST_TIMING") == "1"
+    t0 = time.perf_counter()
     model, data, _ = load_model(a.ckpt_path, device, data_path=a.data_path)
     print(model)
+    t1 = time.perf_counter()
+    if timing:
+        ops.profile_enable(True)                                   # stage events: the rounds apart from PASS 0
     codes, stats = generate_codes(model, data, a.max_rounds, a.chunk_rows)
+    t2 = time.perf_counter()
     print("All indices number: ", len(codes))
     print("Max number of conflicts: ", stats["max_multiplicity"])
     print("Collision Rate", stats["collision_rate"])
     os.makedirs(a.output_dir, exist_ok=True)
     out = os.path.join(a.output_dir, f"{a.dataset}.index.json")
-    write_index_json(codes.to(device), out)                        # formatted on the device
+    if not timing:
+        write_index_json(codes.to(device), out)                    # formatted on the device
+        return out
+    text = ops.index_json_bytes(codes.to(device))                  # what write_index_json does, timed in two parts
+    t3 = time.perf_counter()
+    with open(out, "wb") as fp:
+        fp.write(text)
+    t4 = time.perf_counter()
+    prof = ops.profile_collect()
+    ops.profile_enable(False)
+    rounds_s = sum(ms for tag, (ms, _) in prof.items() if 21 <= tag <= 26) / 1e3      # collision checks + Sinkhorn (GPU time)
+    phases = {"setup_s": t1 - t0, "codes_s": t2 - t1, "pass0_streaming_s": t2 - t1 - rounds_s, "rounds_s": rounds_s,
+              "json_s": t3 - t2, "write_s": t4 - t3}
+    print("generate timing: " + json.dumps(phases), file=sys.stderr)
     return out
+
+
+def _main_sharded(a, world: int) -> str:
+    """``main`` under torchrun: one process per GPU of the box.  Rank r streams its ShardPlan block of the memory-mapped
+    embeddings from the host (in the pieces of the one-GPU run, so PASS 0 gives the same codes), the prefix buckets are
+    exchanged and resolved by their owners (distributed.generate_codes_sharded), and every rank writes its part of the JSON
+    at its offset.  The file and the printed lines are those of the one-GPU run, byte for byte."""
+    import datetime
+    import torch.distributed as dist
+    from .distributed import CudaBackend, ShardPlan, generate_codes_sharded
+    local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    torch.cuda.set_device(local_rank)
+    device = torch.device(f"cuda:{local_rank}")
+    dist.init_process_group("nccl", timeout=datetime.timedelta(seconds=a.dist_timeout))
+    try:
+        rank = dist.get_rank()
+        timing = os.environ.get("LCREC_DIST_TIMING") == "1"
+        t0 = time.perf_counter()
+        model, data, _ = load_model(a.ckpt_path, device, data_path=a.data_path, mmap=True)
+        if rank == 0:
+            print(model)
+        x = data.embeddings
+        n = int(x.shape[0])
+        plan = ShardPlan(n, world)
+        backend = CudaBackend(model, plan.max_count, a.chunk_rows, n_total=n)
+        t1 = time.perf_counter()
+        codes, stats = generate_codes_sharded(backend, x[plan.slice(rank)], plan, rank, a.max_rounds)
+        torch.cuda.synchronize()
+        t2 = time.perf_counter()
+        if rank == 0:
+            print("All indices number: ", n)
+            print("Max number of conflicts: ", stats["max_multiplicity"])
+            print("Collision Rate", stats["collision_rate"])
+            os.makedirs(a.output_dir, exist_ok=True)
+        out = os.path.join(a.output_dir, f"{a.dataset}.index.json")
+        fragment = ops.index_json_bytes(codes, item_base=plan.start(rank), braces=False)      # formatted on this rank's device
+        t3 = time.perf_counter()
+        write_index_json_parts(fragment, out)
+        t4 = time.perf_counter()
+        if timing and rank == 0:
+            phases = {"setup_s": t1 - t0, "codes_s": t2 - t1, "json_s": t3 - t2, "write_s": t4 - t3}
+            phases.update({f"{k}_ms": v for k, v in stats.get("timing_ms", {}).items()})
+            print("generate timing: " + json.dumps(phases), file=sys.stderr)
+        return out
+    finally:
+        dist.destroy_process_group()
 
 
 if __name__ == "__main__":

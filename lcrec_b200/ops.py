@@ -5,6 +5,7 @@ from __future__ import annotations
 import ctypes as C
 from typing import List, Optional, Sequence, Tuple
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -766,21 +767,24 @@ def sinkhorn_groups(resid: torch.Tensor, codebook: torch.Tensor, offsets: torch.
     return int(flags[0].item())
 
 
-def index_json_bytes(codes: torch.Tensor) -> bytes:
+def index_json_bytes(codes: torch.Tensor, item_base: int = 0, braces: bool = True) -> bytes:
     """The `.index.json` text of a CUDA code table (n, L) int64 - the bytes ``json.dump`` writes at
-    generate_indices.py:144-145 - formatted on the device (lcrec_index_json) and copied to the host once."""
+    generate_indices.py:144-145 - formatted on the device (lcrec_index_json_ex) and copied to the host once.
+    ``item_base``: key of the first row; ``braces=False`` leaves out "{" and "}": the fragment of a block of rows, which
+    concatenated with the fragments of the other blocks inside the braces gives the text of the whole table."""
     _need_cuda(codes)
     lib = _lib.load()
     c = codes.detach().to(torch.int64).contiguous()
     n, L = c.shape
+    item_base = int(item_base)
     total = torch.zeros(1, dtype=torch.int64, device=c.device)
     ws = _ws(lib.lcrec_index_json_workspace_bytes(n), c.device)
-    cap = 2 + n * (2 + 1 + 20 + 1 + 2 + 2 + L * (6 + 20 + 2))          # generous upper bound; most of it is never touched
-    if n <= 4_000_000:
-        cap = 2 + n * (2 + 1 + 7 + 1 + 2 + 2 + L * (6 + 20 + 2))
-    out = torch.empty(cap, dtype=torch.uint8, device=c.device)
+    key_digits = max(7, len(str(item_base + n)))                       # digits of the largest key
+    cap = 2 + n * (2 + 1 + key_digits + 1 + 2 + 2 + L * (6 + 20 + 2))  # generous upper bound; most of it is never touched
+    out = torch.empty(max(cap, 1), dtype=torch.uint8, device=c.device)
     with torch.cuda.device(c.device):
-        _lib.check(lib.lcrec_index_json(_p(c), n, L, _p(out), cap, _p(total), _p(ws), ws.numel(), _stream(c)))
+        _lib.check(lib.lcrec_index_json_ex(_p(c), n, L, item_base, int(bool(braces)), _p(out), cap, _p(total), _p(ws),
+                                           ws.numel(), _stream(c)))
     nbytes = int(total.item())
     assert nbytes <= cap
     return out[:nbytes].cpu().numpy().tobytes()
@@ -875,6 +879,25 @@ class Indexer:
             else:
                 _lib.check(self.lib.lcrec_indexer_pass0_ex(self.handle, _p(x2), code, x2.shape[0], int(row_offset),
                                                            _stream(x2)))
+
+    def pass0_host(self, x, n_total: int, row_begin: int = 0) -> None:
+        """PASS 0 of global rows [row_begin, row_begin + n) of an ``n_total``-row job from host memory into table rows
+        [0, n) (lcrec_indexer_pass0_host_ex): bit-identical to those rows of ``run_host`` over all n_total rows.  ``x``:
+        the block as a CPU tensor or ndarray (pinned, pageable or a read-only ``np.memmap`` - read in place, never
+        materialised); fp16 / bf16 stay as they are, other dtypes become an fp32 copy of the block."""
+        if isinstance(x, np.ndarray):
+            if x.dtype not in (np.float16, np.float32) or not x.flags.c_contiguous:
+                x = np.ascontiguousarray(x, dtype=np.float16 if x.dtype == np.float16 else np.float32)
+            ptr, code, n = x.ctypes.data, (1 if x.dtype == np.float16 else 0), int(x.shape[0])
+        else:
+            assert isinstance(x, torch.Tensor) and not x.is_cuda
+            if x.dtype not in (torch.float32,) + _HALF or not x.is_contiguous():
+                x = x.to(x.dtype if x.dtype in _HALF else torch.float32).contiguous()
+            ptr, code, n = x.data_ptr(), DTYPE_CODES[x.dtype], int(x.shape[0])
+        with torch.cuda.device(self.device):
+            st = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+            _lib.check(self.lib.lcrec_indexer_pass0_host_ex(self.handle, C.c_void_p(ptr), code, int(n_total), int(row_begin), n,
+                                                            st))
 
     def round(self, n: int) -> dict:
         counts = (C.c_int64 * 4)()
