@@ -195,7 +195,9 @@ int lcrec_bn_backward_apply(const float* y, const float* gy, const float* out, i
 
 /* ---- a10 (training): reconstruction loss of RQVAE.compute_loss (index/models/rqvae.py:74-85) ---------------------------
  * loss (1 fp32, device) = mean over `total` = n * in_dim elements of (out - x)^2 (loss_type 0, F.mse_loss) or |out - x|
- * (1, F.l1_loss); fp64 partial sums in a fixed order.  backward: grad = (*upstream, or 1 when NULL) * d loss / d out. */
+ * (1, F.l1_loss); fp64 partial sums in a fixed order.  backward: grad = (*upstream, or 1 when NULL) * d loss / d out.
+ * out / x / grad need only 4-byte (fp32) alignment: float4 accesses are used when all of them are 16-byte aligned, and
+ * the result is the same bit for bit either way. */
 int64_t lcrec_recon_loss_workspace_bytes(int64_t total);
 int lcrec_recon_loss(const float* out, const float* x, int64_t total, int loss_type, float* loss, void* ws, int64_t ws_bytes,
                      void* stream);

@@ -79,7 +79,7 @@ bn_apply_kernel(const float* __restrict__ y, const double* __restrict__ sums, in
   for (int s = 0; s < splits; ++s) { sa += sums[((size_t)s * 2 + 0) * C + c]; sb += sums[((size_t)s * 2 + 1) * C + c]; }
   const double m = sa / (double)n_total;
   double var = sb / (double)n_total - m * m;                 // biased variance (what normalises the batch)
-  var = var > 0.0 ? var : 0.0;
+  var = var < 0.0 ? 0.0 : var;                               // NaN passes (inf in a channel: inf - inf), like torch
   const float mu = (float)m;
   const float is = (float)(1.0 / sqrt(var + (double)eps));
   if (blockIdx.y == 0 && rl == 0) {
@@ -131,9 +131,26 @@ bn_backward_apply_kernel(const float* __restrict__ y, const float* __restrict__ 
 }
 
 // ---- reconstruction loss
+// VEC: every pointer is 16-byte aligned and groups of 4 elements move as float4; otherwise the same groups are loaded and
+// stored one float at a time.  The arithmetic is the same either way, so an offset view gives the aligned copy's values.
 constexpr int kLossThreads = 256;
 constexpr int kLossPerCta = kLossThreads * 16;
 
+template <bool VEC>
+__device__ __forceinline__ float4 ld4(const float* p) {
+  if (VEC) return *reinterpret_cast<const float4*>(p);
+  return make_float4(p[0], p[1], p[2], p[3]);
+}
+
+template <bool VEC>
+__device__ __forceinline__ void st4(float* p, float4 v) {
+  if (VEC) { *reinterpret_cast<float4*>(p) = v; return; }
+  p[0] = v.x; p[1] = v.y; p[2] = v.z; p[3] = v.w;
+}
+
+static bool aligned16(const void* p) { return p == nullptr || (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+template <bool VEC>
 __global__ void __launch_bounds__(kLossThreads)
 recon_partial_kernel(const float* __restrict__ out, const float* __restrict__ x, int64_t total, int l1, double* __restrict__ partial) {
   __shared__ double red[kLossThreads / 32];
@@ -143,7 +160,7 @@ recon_partial_kernel(const float* __restrict__ out, const float* __restrict__ x,
     for (int u = 0; u < 4; ++u) {
       const int64_t j = i + (int64_t)u * kLossThreads * 4;
       if (j + 3 < total) {
-        const float4 a = *reinterpret_cast<const float4*>(out + j), b = *reinterpret_cast<const float4*>(x + j);
+        const float4 a = ld4<VEC>(out + j), b = ld4<VEC>(x + j);
         const float d0 = a.x - b.x, d1 = a.y - b.y, d2 = a.z - b.z, d3 = a.w - b.w;
         const float t = l1 ? (fabsf(d0) + fabsf(d1)) + (fabsf(d2) + fabsf(d3)) : fmaf(d0, d0, d1 * d1) + fmaf(d2, d2, d3 * d3);
         s += (double)t;
@@ -179,6 +196,7 @@ __global__ void recon_final_kernel(const double* __restrict__ partial, int n_par
 }
 
 // grad = upstream * d mean(loss) / d out:  mse: 2 (out - x) / total;  l1: sign(out - x) / total
+template <bool VEC>
 __global__ void __launch_bounds__(kLossThreads)
 recon_backward_kernel(const float* __restrict__ out, const float* __restrict__ x, int64_t total, int l1,
                       const float* __restrict__ upstream, float inv_total, float* __restrict__ grad) {
@@ -186,7 +204,7 @@ recon_backward_kernel(const float* __restrict__ out, const float* __restrict__ x
   const float k = (l1 ? 1.f : 2.f) * inv_total * up;
   for (int64_t i = ((int64_t)blockIdx.x * kLossThreads + threadIdx.x) * 4; i < total; i += (int64_t)gridDim.x * kLossThreads * 4) {
     if (i + 3 < total) {
-      const float4 a = *reinterpret_cast<const float4*>(out + i), b = *reinterpret_cast<const float4*>(x + i);
+      const float4 a = ld4<VEC>(out + i), b = ld4<VEC>(x + i);
       float4 g;
       if (l1) {
         g.x = k * (float)((a.x > b.x) - (a.x < b.x)); g.y = k * (float)((a.y > b.y) - (a.y < b.y));
@@ -194,7 +212,7 @@ recon_backward_kernel(const float* __restrict__ out, const float* __restrict__ x
       } else {
         g.x = k * (a.x - b.x); g.y = k * (a.y - b.y); g.z = k * (a.z - b.z); g.w = k * (a.w - b.w);
       }
-      *reinterpret_cast<float4*>(grad + i) = g;
+      st4<VEC>(grad + i, g);
     } else {
       for (int64_t q = i; q < total; ++q) {
         const float d = out[q] - x[q];
@@ -276,7 +294,8 @@ extern "C" int64_t lcrec_recon_loss_workspace_bytes(int64_t total) {
   return arena_need(ctas * 8);
 }
 
-// loss (1 fp32, device) = mean over `total` elements of (out - x)^2 (loss_type 0, F.mse_loss) or |out - x| (1, F.l1_loss)
+// loss (1 fp32, device) = mean over `total` elements of (out - x)^2 (loss_type 0, F.mse_loss) or |out - x| (1, F.l1_loss).
+// Any 4-byte-aligned out / x (an offset view included); 16-byte-aligned pointers take the float4 loads.
 extern "C" int lcrec_recon_loss(const float* out, const float* x, int64_t total, int loss_type, float* loss, void* ws,
                                 int64_t ws_bytes, void* stream) {
   LC_ARG(total >= 1 && out && x && loss && (loss_type == 0 || loss_type == 1));
@@ -285,20 +304,27 @@ extern "C" int lcrec_recon_loss(const float* out, const float* x, int64_t total,
   Arena ar(ws, ws_bytes);
   double* partial = ar.take<double>(ctas);
   if (!ar.ok()) { set_error("recon_loss: workspace too small"); return LCREC_ERR_NOMEM; }
-  recon_partial_kernel<<<ctas, kLossThreads, 0, (cudaStream_t)stream>>>(out, x, total, loss_type, partial);
+  if (aligned16(out) && aligned16(x))
+    recon_partial_kernel<true><<<ctas, kLossThreads, 0, (cudaStream_t)stream>>>(out, x, total, loss_type, partial);
+  else
+    recon_partial_kernel<false><<<ctas, kLossThreads, 0, (cudaStream_t)stream>>>(out, x, total, loss_type, partial);
   LC_LAUNCH_CHECK("recon_partial_kernel");
   recon_final_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(partial, ctas, 1.0 / (double)total, loss);
   LC_LAUNCH_CHECK("recon_final_kernel");
   return LCREC_OK;
 }
 
-// grad = (*upstream, or 1 when NULL) * d loss / d out
+// grad = (*upstream, or 1 when NULL) * d loss / d out; any 4-byte-aligned out / x / grad, float4 accesses when all three are 16-byte aligned
 extern "C" int lcrec_recon_loss_backward(const float* out, const float* x, int64_t total, int loss_type, const float* upstream,
                                          float* grad, void* stream) {
   LC_ARG(total >= 1 && out && x && grad && (loss_type == 0 || loss_type == 1));
   LC_TRY(lcrec_device_check());
   const int ctas = (int)std::max<int64_t>(1, std::min<int64_t>(ceil_div(total, kLossThreads * 4 * 4), (int64_t)num_sms() * 16));
-  recon_backward_kernel<<<ctas, kLossThreads, 0, (cudaStream_t)stream>>>(out, x, total, loss_type, upstream, (float)(1.0 / (double)total), grad);
+  const float inv_total = (float)(1.0 / (double)total);
+  if (aligned16(out) && aligned16(x) && aligned16(grad))
+    recon_backward_kernel<true><<<ctas, kLossThreads, 0, (cudaStream_t)stream>>>(out, x, total, loss_type, upstream, inv_total, grad);
+  else
+    recon_backward_kernel<false><<<ctas, kLossThreads, 0, (cudaStream_t)stream>>>(out, x, total, loss_type, upstream, inv_total, grad);
   LC_LAUNCH_CHECK("recon_backward_kernel");
   return LCREC_OK;
 }

@@ -69,6 +69,8 @@ class _BnReluFn(torch.autograd.Function):
     def forward(ctx, y, gamma, beta, bn, relu: bool):
         sync = getattr(bn, "lcrec_sync", None)
         group, n_total = sync if sync is not None else (None, None)
+        if (n_total if n_total is not None else y.shape[0]) == 1:   # F.batch_norm's check, on the global batch
+            raise ValueError(f"Expected more than 1 value per channel when training, got input size {y.size()}")
         factor = 0.0
         rm = rv = None
         if bn.track_running_stats and bn.running_mean is not None:
